@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py - CTR inferences/s of the DIN forward path (BASELINE.json configs[2]).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 What is scored: DIN ranking instances (T=50, E=32, MovieLens-20M-shaped vocabularies, synthetic
 Zipf inputs, seeded random-init weights of the reference architecture) in batches of `--batch`
@@ -41,6 +41,9 @@ NVLink).  Each rank binds to the CPUs of its GPU's NUMA node before it allocates
 `--workload cfg5_din` (10^8-row table) launches directly instead of replaying a graph (`--graph`
 restores the replay; why: DESIGN.md section 6).  stdout carries the one JSON line and nothing else;
 an outer `timeout` (SIGTERM) makes the script dump its Python stacks to stderr first.
+`--dump-outputs DIR` writes the scores of the last timed step to DIR/scores.npy ([batches, rows], float32;
+`scores_rank<r>.npy` per rank with N > 1): the inputs are seeded, so two builds run with the same arguments
+can be compared output for output.
 """
 from __future__ import annotations
 
@@ -65,6 +68,7 @@ for _k, _v in (("OMP_WAIT_POLICY", "PASSIVE"), ("GOMP_SPINCOUNT", "0"), ("OMP_PR
 METRIC = "CTR inferences/sec (DIN, batch=4096, hist_len=50)"
 WORKLOAD = "cfg3_din"
 L2_BYTES = 126 * 1024 * 1024
+DUMP_BYTES = 64 << 20                   # --dump-outputs: at most this much in all, a seeded sample of batches above
 DTYPE = "bf16x3 (fp32 accumulate)"      # every MMA operand is split hi + lo, three products, fp32 accumulators
 
 # BASELINE.json configs -> (default rows per GPU per launch, metric label).  cfg3_din is the
@@ -122,7 +126,11 @@ def parse_args(argv=None):
                     help="distribution of the history ids (default: uniform for cfg 5 - the L2-defeating worst case "
                          "BASELINE.md asks for - Zipf(1.05) otherwise)")
     ap.add_argument("--cpu-seconds", type=float, default=10.0)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the scores of the last timed step to DIR/scores.npy")
     args = ap.parse_args(argv)
+    if args.dump_outputs and (args.impl != "ours" or args.gather == "fused"):
+        ap.error("--dump-outputs writes the scores of --impl ours without --gather fused")
     if args.batch is None:
         args.batch = WORKLOADS[args.workload][0]
     # cfg 5 launches directly: CUDA-graph replays of din_rt64_kernel on the 10^8-row table did not finish in
@@ -479,6 +487,19 @@ def tile_encoded(enc, reps, rng):
                         cat(enc.movie_genre), cat(enc.user_genre), cat(enc.numerics))
 
 
+def dump_outputs(directory, name, scores, limit):
+    """Write `scores` ([batches, rows], on the device) to directory/name.npy as float32: all of it, or when that
+    exceeds `limit` bytes a seeded sample of whole batches, the same batches on every run."""
+    import torch
+    os.makedirs(directory, exist_ok=True)
+    n, rows = scores.shape
+    keep = min(n, max(1, limit // (4 * rows)))
+    if keep < n:
+        idx = np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+        scores = scores[torch.from_numpy(idx).to(scores.device)]
+    np.save(os.path.join(directory, name + ".npy"), scores.float().cpu().numpy())
+
+
 def run_ours(args):
     rank, local_rank, world = dist_env()
     prev_affinity, numa_note = (None, "not bound (--no-numa-bind)") if args.no_numa_bind \
@@ -658,6 +679,8 @@ def run_ours(args):
         torch.cuda.synchronize()
         ms = ev0.elapsed_time(ev1)
     model.status()                                     # no id was out of range
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, "scores" if world == 1 else "scores_rank%d" % rank, out, DUMP_BYTES // world)
     if S > 1:
         model.set_sm_limit(0)                          # the host legs below are single launches again
 

@@ -9,7 +9,6 @@ if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
 GOLDEN = os.path.join(ROOT, "tests", "golden")
-REFERENCE_WEBROOT = "/root/reference/src/main/resources/webroot/"
 
 
 def pytest_configure(config):

@@ -1,6 +1,6 @@
-"""Golden vectors from the reference's own serialised graphs (run where /root/reference exists):
+"""Golden vectors from the reference's own serialised graphs:
 
-    python tests/golden/make_savedmodel_graph_vectors.py
+    python tests/golden/make_savedmodel_graph_vectors.py <SparrowRecSys checkout>
 
 For each shipped export (`modeldata/neuralcf/{002,001}`, `modeldata/MLPRec/005`) `oracle/savedmodel_graph.py`
 reads `saved_model.pb`, follows `serving_default` to the `__inference__wrapped_model_*` function TensorFlow wrote,
@@ -21,18 +21,18 @@ sys.path.insert(0, os.path.dirname(os.path.dirname(HERE)))
 from oracle import savedmodel_graph as G                               # noqa: E402
 from sparrowrecsys_b200 import bundle, features                        # noqa: E402
 
-REF = "/root/reference/src/main/resources/webroot/"
 EXPORTS = {"neuralcf_002": "modeldata/neuralcf/002", "neuralcf_001": "modeldata/neuralcf/001",
            "mlprec_005": "modeldata/MLPRec/005"}
 
 
-def vectors():
+def vectors(webroot):
+    """`webroot`: a directory holding the reference's `modeldata/` (its `src/main/resources/webroot`)."""
     rows = features.load_samples_csv(os.path.join(HERE, "samples_head.csv"))
     movie = np.concatenate([np.asarray(rows["movieId"]), [52, 53]]).astype(np.int64)
     user = np.concatenate([np.asarray(rows["userId"]), [10351, 10351]]).astype(np.int64)
     out = {}
     for name, rel in EXPORTS.items():
-        g = G.ServingGraph(REF + rel, bundle.read_variables)
+        g = G.ServingGraph(os.path.join(webroot, rel), bundle.read_variables)
         feeds = {ph: np.zeros(len(movie), np.int64) for ph in g.placeholders.values()}   # unused inputs of MLPRec/005
         feeds["movieId"], feeds["userId"] = movie, user
         y = g.run(feeds).reshape(-1)
@@ -53,7 +53,7 @@ def vectors():
     # categorical_column_with_vocabulary_list do - the semantics every other graph of the oracle rests on
     for name, rel in (("mlprec_001", "modeldata/MLPRec/001"), ("mlprec_002", "modeldata/MLPRec/002"),
                       ("mlprec_003", "modeldata/MLPRec/003"), ("mlprec_004", "modeldata/MLPRec/004")):
-        g = G.ServingGraph(REF + rel, bundle.read_variables)
+        g = G.ServingGraph(os.path.join(webroot, rel), bundle.read_variables)
         voc = g.vocabulary_tables()
         casts = sorted(n.name.split("/")[-2] for n in g.fn.nodes.values()
                        if n.op == "Cast" and n.data_inputs()[0] in g.placeholders)
@@ -78,6 +78,8 @@ def vectors():
 
 
 if __name__ == "__main__":
+    if len(sys.argv) != 2:
+        sys.exit(__doc__)
     with open(os.path.join(HERE, "savedmodel_graph_vectors.json"), "w") as f:
-        json.dump(vectors(), f, indent=0)
+        json.dump(vectors(os.path.join(sys.argv[1], "src", "main", "resources", "webroot")), f, indent=0)
     print("wrote savedmodel_graph_vectors.json")

@@ -84,3 +84,21 @@ def test_stdout_of_the_reference_arm_is_one_json_line():
     assert d["impl"] == "reference" and d["unit"] == "inferences/s" and d["value"] > 0
     assert d["e2e"]["h2d_bytes_per_step"] == 0 and d["cpu_baseline"]["kind"] == "port"
     assert d["dtype"] == "f32" and d["higher_is_better"] is True
+
+
+def test_dumped_outputs_are_bounded_and_the_same_batches_every_run(tmp_path):
+    """--dump-outputs: the whole [batches, rows] score array when it fits the limit, otherwise the same seeded
+    sample of whole batches on every run, so that two builds can be compared output for output."""
+    import pytest
+    import torch
+    import bench
+    scores = torch.arange(64 * 32, dtype=torch.float32).reshape(64, 32)
+    bench.dump_outputs(str(tmp_path / "all"), "scores", scores, 1 << 20)
+    assert np.array_equal(np.load(tmp_path / "all" / "scores.npy"), scores.numpy())
+    for run in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / run), "scores", scores, 10 * 32 * 4)
+    a, b = np.load(tmp_path / "a" / "scores.npy"), np.load(tmp_path / "b" / "scores.npy")
+    assert a.dtype == np.float32 and a.shape == (10, 32) and np.array_equal(a, b)
+    assert len({int(r[0]) // 32 for r in a}) == 10 and all(np.array_equal(r, r[0] + np.arange(32)) for r in a)
+    with pytest.raises(SystemExit):
+        bench.parse_args(["--impl", "reference", "--dump-outputs", str(tmp_path)])

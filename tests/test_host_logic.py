@@ -147,7 +147,14 @@ def test_abi_library_exports_every_declared_symbol():
     assert set(declared) == set(_lib.EXPORTS)
     assert lib.srs_abi_version() == _lib.ABI_VERSION == 3
     assert lib.srs_num_slots() >= 2
-    assert lib.srs_launch_count() == 0
+    # loading and querying the library launches nothing; checked in a fresh process because the launch counter is
+    # per process and GPU tests of the same session may have launched before this one
+    import subprocess
+    import sys
+    r = subprocess.run([sys.executable, "-c", "import sys; sys.path.insert(0, %r); from sparrowrecsys_b200 import _lib; "
+                        "lib = _lib.load(); lib.srs_abi_version(); lib.srs_num_slots(); print(lib.srs_launch_count())"
+                        % ROOT], cwd=ROOT, capture_output=True, text=True, timeout=300)
+    assert r.returncode == 0 and r.stdout.strip() == "0", r.stdout + r.stderr
 
 
 def test_struct_layouts_match_header():

@@ -1,13 +1,15 @@
 """Pin the oracle: shipped trained weights of the reference on the bundled test rows
 must reproduce the known answers recorded in SURVEY.md section 8c (computed there by
 an independent numpy restatement of the graph; TensorFlow itself cannot run here)."""
+import gzip
+import hashlib
 import json
 import os
 
 import numpy as np
 import pytest
 
-from conftest import GOLDEN, REFERENCE_WEBROOT, load_golden_weights
+from conftest import GOLDEN, load_golden_weights
 from oracle import ctr_oracle as O
 from sparrowrecsys_b200.spec import default_spec
 
@@ -21,6 +23,21 @@ KNOWN = {
     "mlprec_005": [0.5534312, 0.21570465, 0.09113927, 0.37527242, 0.22620608, 0.5138782,
                    0.43187657, 0.9393208],
 }
+
+
+@pytest.fixture(scope="module")
+def webroot(tmp_path_factory):
+    """The reference's model exports as tests/golden/make_reference_exports.py stored them, unpacked in the layout of
+    its `src/main/resources/webroot/modeldata`; returns the directory that holds `modeldata/`."""
+    root = tmp_path_factory.mktemp("webroot")
+    src = os.path.join(GOLDEN, "modeldata")
+    for dirpath, _, files in os.walk(src):
+        for name in files:
+            dst = root / "modeldata" / os.path.relpath(os.path.join(dirpath, name[:-len(".gz")]), src)
+            dst.parent.mkdir(parents=True, exist_ok=True)
+            with gzip.open(os.path.join(dirpath, name), "rb") as f:
+                dst.write_bytes(f.read())
+    return str(root) + os.sep
 
 
 def test_head_rows_are_the_surveyed_rows(head_rows):
@@ -63,31 +80,31 @@ def test_full_file_stats_recorded():
     assert abs(s["roc_auc"] - 0.73208) < 1e-5
 
 
-@pytest.mark.skipif(not os.path.isdir(REFERENCE_WEBROOT), reason="reference checkout not present")
-def test_bundle_reader_matches_fixture():
+def test_bundle_reader_matches_fixture(webroot):
     """The TF-free bundle reader on the real SavedModel dirs equals the committed fixture."""
     from sparrowrecsys_b200 import bundle
-    W = bundle.load_neuralcf(REFERENCE_WEBROOT + "modeldata/neuralcf/002")
+    W = bundle.load_neuralcf(webroot + "modeldata/neuralcf/002")
     G = load_golden_weights("neuralcf_002")
     for k in ("movieId_embedding", "dense_0/kernel", "dense_0/bias", "dense_1/kernel",
               "dense_2/kernel", "dense_2/bias"):
         assert np.array_equal(W[k], G[k]), k
     nz = np.flatnonzero(np.abs(G["userId_embedding"]).sum(axis=1))
     assert np.array_equal(W["userId_embedding"][nz], G["userId_embedding"][nz])
-    idx = bundle.read_index(REFERENCE_WEBROOT + "modeldata/neuralcf/002/variables/variables.index")
+    idx = bundle.read_index(webroot + "modeldata/neuralcf/002/variables/variables.index")
     e = idx["layer_with_weights-2/kernel/.ATTRIBUTES/VARIABLE_VALUE"]
     assert (e["shape"], e["offset"]) == ((20, 10), 1240080)       # SURVEY.md 8c offsets
-    W5 = bundle.load_twotowers(REFERENCE_WEBROOT + "modeldata/MLPRec/005")
+    W5 = bundle.load_twotowers(webroot + "modeldata/MLPRec/005")
     assert W5["item_dense_0/kernel"].shape == (10, 10)
 
 
-@pytest.mark.skipif(not os.path.isdir(REFERENCE_WEBROOT), reason="reference checkout not present")
 def test_head_fixture_is_prefix_of_reference_file():
-    with open(REFERENCE_WEBROOT + "sampledata/testSamples.csv", "rb") as f:
-        ref = f.read(200000)
+    """samples_head.csv is byte for byte the start of the reference's testSamples.csv (length and SHA-256 of that
+    prefix recorded in reference_files.json)."""
+    with open(os.path.join(GOLDEN, "reference_files.json")) as f:
+        ref = json.load(f)["sampledata/testSamples.csv"]
     with open(os.path.join(GOLDEN, "samples_head.csv"), "rb") as f:
         head = f.read()
-    assert ref.startswith(head)
+    assert len(head) == ref["prefix_bytes"] and hashlib.sha256(head).hexdigest() == ref["prefix_sha256"]
 
 
 # ---- the reference's own serialised graphs (tests/golden/make_savedmodel_graph_vectors.py) ----------------
@@ -187,21 +204,20 @@ def test_feature_column_semantics_read_off_the_older_exports():
     assert O.genre_index(f, "movieGenre1").tolist() == [0, 18, -1, -1, 1]
 
 
-@pytest.mark.skipif(not os.path.isdir(REFERENCE_WEBROOT), reason="reference checkout not present")
-def test_identity_column_edge_cases_of_the_serialised_graph():
+def test_identity_column_edge_cases_of_the_serialised_graph(webroot):
     """What the reference's graph itself does with odd ids: an id >= num_buckets trips the graph's own assert (our
     ValueError / SRS_ERR_RANGE), the last valid id works, and -1 is the column's "missing" value: its embedding is
     the zero vector (we reject -1 instead: INTEGRATION.md, error table)."""
     from oracle import savedmodel_graph as SG
     from sparrowrecsys_b200 import bundle
-    g = SG.ServingGraph(REFERENCE_WEBROOT + "modeldata/neuralcf/002", bundle.read_variables)
+    g = SG.ServingGraph(webroot + "modeldata/neuralcf/002", bundle.read_variables)
     with pytest.raises(ValueError):
         g.run({"movieId": np.array([5, 1001]), "userId": np.array([7, 7])})
     with pytest.raises(ValueError):
         g.run({"movieId": np.array([5, 5]), "userId": np.array([7, 30001])})
     ok = g.run({"movieId": np.array([5, 1000]), "userId": np.array([7, 30000])})
     assert ok.shape == (2, 1)
-    W = bundle.load_neuralcf(REFERENCE_WEBROOT + "modeldata/neuralcf/002")
+    W = bundle.load_neuralcf(webroot + "modeldata/neuralcf/002")
     missing = g.run({"movieId": np.array([-1]), "userId": np.array([7])})
     Wz = dict(W)
     Wz["movieId_embedding"] = W["movieId_embedding"].copy()
@@ -212,30 +228,30 @@ def test_identity_column_edge_cases_of_the_serialised_graph():
                           g.run({"movieId": np.array([3, 9]), "userId": np.array([7, 8])}, full=False))
 
 
-@pytest.mark.skipif(not os.path.isdir(REFERENCE_WEBROOT), reason="reference checkout not present")
-def test_graph_vectors_regenerate_from_the_reference_exports():
+def test_graph_vectors_regenerate_from_the_reference_exports(webroot):
     import importlib.util
     spec = importlib.util.spec_from_file_location("mk", os.path.join(GOLDEN, "make_savedmodel_graph_vectors.py"))
     mk = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(mk)
-    fresh = json.loads(json.dumps(mk.vectors()))
+    fresh = json.loads(json.dumps(mk.vectors(webroot)))
     assert fresh == _graph_vectors()
 
 
-@pytest.mark.skipif(not os.path.isdir(REFERENCE_WEBROOT), reason="reference checkout not present")
-def test_whole_test_file_through_the_serialised_graph():
-    """All 22 440 rows of the reference's testSamples.csv through the serialised neuralcf/002 graph: the oracle agrees
-    row by row, and the accuracy / ROC-AUC recorded in full_file_stats.json (SURVEY.md 8c) are the graph's."""
+def test_whole_test_file_through_the_serialised_graph(webroot):
+    """All 22 440 rows of the reference's testSamples.csv through the serialised neuralcf/002 graph
+    (full_file_graph.npz): the accuracy / ROC-AUC recorded in full_file_stats.json (SURVEY.md 8c) are the graph's,
+    and on the stored sample of rows the graph, evaluated again here, and the oracle agree with it row by row."""
     from oracle import savedmodel_graph as SG
     from sparrowrecsys_b200 import bundle
-    from sparrowrecsys_b200.features import load_samples_csv
-    full = load_samples_csv(REFERENCE_WEBROOT + "sampledata/testSamples.csv")
-    g = SG.ServingGraph(REFERENCE_WEBROOT + "modeldata/neuralcf/002", bundle.read_variables)
-    pg = g.run({"movieId": np.asarray(full["movieId"]), "userId": np.asarray(full["userId"])})[:, 0]
-    W = bundle.load_neuralcf(REFERENCE_WEBROOT + "modeldata/neuralcf/002")
-    po = O.predict(default_spec("neuralcf"), W, full)[:, 0]
-    assert len(pg) == 22440 and np.abs(pg - po).max() <= 5e-7
-    lab = np.asarray(full["label"])
+    z = np.load(os.path.join(GOLDEN, "full_file_graph.npz"))
+    pg, lab, rows = z["prob"], z["label"], z["rows"]
+    sample = {"movieId": z["movieId"], "userId": z["userId"]}
+    g = SG.ServingGraph(webroot + "modeldata/neuralcf/002", bundle.read_variables)
+    ps = g.run(sample)[:, 0]
+    W = bundle.load_neuralcf(webroot + "modeldata/neuralcf/002")
+    po = O.predict(default_spec("neuralcf"), W, sample)[:, 0]
+    assert len(pg) == len(lab) == 22440 and len(rows) == 2048
+    assert np.abs(ps - pg[rows]).max() <= 5e-7 and np.abs(po - pg[rows]).max() <= 5e-7
     with open(os.path.join(GOLDEN, "full_file_stats.json")) as f:
         s = json.load(f)
     assert abs(float(((pg > 0.5) == (lab == 1)).mean()) - s["accuracy"]) < 1e-9
