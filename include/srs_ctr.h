@@ -249,6 +249,43 @@ int srs_cosine_scores_device(const float* query, const float* cands, int32_t n, 
 int srs_topk_device(const float* scores, int32_t n, int32_t k, int32_t* top_idx,
                     float* top_scores, int32_t device, void* stream);
 
+/* ---- Candidate retrieval: exact top-k over an item index resident in HBM.  Replaces the recall stage
+ * in front of the rankers: SimilarMovieProcess.retrievalCandidatesByEmbedding (SimilarMovieProcess.java:91-112,
+ * which scores the whole catalog by Embedding.calculateSimilarity) and the fixed candidate list of
+ * RecForYouProcess.getRecList (RecForYouProcess.java:34-35, getMovies(800, "rating")); the output feeds
+ * srs_rank_user_host.  Unlike SimilarMovieProcess.java:104 (an ascending sort, which keeps the LEAST similar
+ * movies) the result is the most similar first, as the ranker (SimilarMovieProcess.java:135) intends.
+ *
+ * srs_index_create: an index over n items [n][dim] float32 (1 <= n < 2^31, 1 <= dim <= 128).  The library
+ * keeps a bf16 scan copy (cosine: of the unit-length rows), per-row norms, and the float32 rows for exact
+ * rescoring: copied from host memory (SRS_HOST), or used in place when `items` is a device pointer on
+ * `device` (SRS_DEVICE_BORROWED; it must outlive the index).
+ * Scores: SRS_DOT = float32 fmaf chain over k = 0..dim-1; SRS_COSINE = Embedding.calculateSimilarity
+ * (online/model/Embedding.java:33-47), bit for bit what srs_cosine_scores_device gives for the pair.  A zero
+ * row's cosine is 0/0 = NaN and, as in the reference's Double ordering, ranks first. */
+enum srs_metric { SRS_DOT = 0, SRS_COSINE = 1 };
+typedef struct srs_index srs_index;
+int srs_index_create(const float* items, int64_t n, int32_t dim, int32_t metric, int32_t location,
+                     int32_t device, srs_index** out);
+void srs_index_destroy(srs_index* index);
+
+/* Search q queries [q][dim] (dim must equal the index's), 1 <= k <= 1024, `exclude` [q] an item position
+ * per query to leave out (-1 = none; NULL = none for every query).  For each query: top_pos [q][k] and
+ * top_scores [q][k] receive the best min(k, eligible) positions, best first, in the order of
+ * srs_topk_device (descending score, NaN first, -0.0 after 0.0, equal scores by lower position), and their
+ * exact scores; unused slots get position -1 and score 0.  No q x n score matrix is formed and the result
+ * does not depend on timing.
+ * srs_index_search_device: device pointers, queued on `stream`; it synchronises `stream` once per block of
+ * 256 queries, and again for each extra pass a query whose candidates overflow needs.  Calls on one index
+ * are serialised, also across streams: a search waits on the device for the previous search of the same
+ * index to finish (its working lists are per index).
+ * srs_index_search_host: host pointers, synchronous.
+ * An exclude position outside -1..n-1 is SRS_ERR_INVALID. */
+int srs_index_search_device(srs_index* index, const float* queries, int32_t q, int32_t dim, int32_t k,
+                            const int32_t* exclude, int32_t* top_pos, float* top_scores, void* stream);
+int srs_index_search_host(srs_index* index, const float* queries, int32_t q, int32_t dim, int32_t k,
+                          const int32_t* exclude, int32_t* top_pos, float* top_scores);
+
 /* One ranking call from host buffers: H2D of the candidate batch, forward kernel, ranking
  * kernel, D2H of the min(k, B) best positions and scores only.  Replaces
  * RecForYouProcess.ranker (:69-95) with model "nerualcf" followed by getRecList's subList:

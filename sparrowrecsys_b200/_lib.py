@@ -14,6 +14,7 @@ SRS_OK = 0
 SRS_ERR_INVALID, SRS_ERR_MISSING, SRS_ERR_SHAPE = -1, -2, -3
 SRS_ERR_CUDA, SRS_ERR_RANGE, SRS_ERR_NOMEM = -4, -5, -6
 SRS_HOST, SRS_DEVICE_BORROWED = 0, 1
+SRS_DOT, SRS_COSINE = 0, 1
 ABI_VERSION = 3
 
 
@@ -42,7 +43,8 @@ EXPORTS = ("srs_abi_version", "srs_last_error", "srs_model_create", "srs_model_c
            "srs_cosine_scores_device", "srs_topk_device", "srs_rank_host", "srs_gather_create", "srs_gather_export",
            "srs_gather_connect", "srs_gather_destroy", "srs_predict_device_gather", "srs_gather_wait",
            "srs_gather_scores", "srs_gather_copy_scores", "srs_model_set_movie_features", "srs_rank_user_host",
-           "srs_selftest_umma", "srs_debug_din_trace", "srs_debug_din_timeline", "srs_debug_umma_bench")
+           "srs_selftest_umma", "srs_debug_din_trace", "srs_debug_din_timeline", "srs_debug_umma_bench",
+           "srs_index_create", "srs_index_destroy", "srs_index_search_device", "srs_index_search_host")
 
 _lib = None
 
@@ -150,6 +152,17 @@ def load():
     lib.srs_selftest_umma.restype = C.c_int
     lib.srs_selftest_umma.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32,
                                       C.c_int32, C.c_int32]
+    lib.srs_index_create.restype = C.c_int
+    lib.srs_index_create.argtypes = [C.c_void_p, C.c_int64, C.c_int32, C.c_int32, C.c_int32, C.c_int32,
+                                     C.POINTER(C.c_void_p)]
+    lib.srs_index_destroy.restype = None
+    lib.srs_index_destroy.argtypes = [C.c_void_p]
+    lib.srs_index_search_device.restype = C.c_int
+    lib.srs_index_search_device.argtypes = [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_void_p,
+                                            C.c_void_p, C.c_void_p, C.c_void_p]
+    lib.srs_index_search_host.restype = C.c_int
+    lib.srs_index_search_host.argtypes = [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_void_p,
+                                          C.c_void_p, C.c_void_p]
     if lib.srs_abi_version() != ABI_VERSION:
         raise ImportError("libsrs_ctr.so ABI version %d != %d" % (lib.srs_abi_version(), ABI_VERSION))
     _lib = lib

@@ -59,6 +59,15 @@ int fail(int code, const char* fmt, ...) {
   return code;
 }
 
+}  // namespace
+
+namespace srs {
+// srs_last_error() of the entry points defined outside this file (retrieve.cu)
+int report_error(int code, const char* msg) { return fail(code, "%s", msg); }
+}  // namespace srs
+
+namespace {
+
 // Kernel-variant options of the model being created: "key=value;key=value" handed to
 // srs_model_create_ex (keys: din_impl, embmlp_impl, deepfm_impl, zero_copy_scores).  The environment variables SRS_<KEY> remain as a tuning override of last resort.
 thread_local std::string g_create_opts;

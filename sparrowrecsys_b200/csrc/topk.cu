@@ -14,6 +14,7 @@
 // n <= 4096 (the reference ranks 800 candidates), shared-memory chunks plus global
 // compare-exchange steps above that.
 #include "kernels.h"
+#include "rank.cuh"
 
 namespace srs {
 
@@ -21,26 +22,6 @@ namespace {
 
 constexpr int kSortChunk = 4096;            // keys one CTA sorts in shared memory (32 KB)
 constexpr int kSortThreads = 1024;
-constexpr uint64_t kPadKey = ~0ull;     // sorts after every real key
-
-__device__ __forceinline__ uint64_t rank_key(float s, uint32_t i) {
-  uint32_t u = __float_as_uint(s);
-  if (s != s) u = 0xFFFFFFFFu;                                    // NaN: greatest
-  else u = (u & 0x80000000u) ? ~u : (u | 0x80000000u);            // monotone float -> uint
-  return ((uint64_t)(~u) << 32) | i;                              // ascending key = descending score
-}
-
-// compare-exchange of the pair (i, i | j) for the bitonic stage of width k
-__device__ __forceinline__ void cmpx(uint64_t& a, uint64_t& b, bool ascending) {
-  if ((a > b) == ascending) {
-    const uint64_t t = a; a = b; b = t;
-  }
-}
-
-// position of the t-th pair's lower element: t with a zero inserted at bit log2(j)
-__device__ __forceinline__ uint32_t pair_lo(uint32_t t, uint32_t j) {
-  return ((t & ~(j - 1)) << 1) | (t & (j - 1));
-}
 
 // n <= NP <= kSortChunk: the whole ranking in one CTA.
 __global__ void __launch_bounds__(kSortThreads)

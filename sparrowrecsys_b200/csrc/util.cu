@@ -1,5 +1,6 @@
 // util.cu - small device utilities around the forward path.
 #include "kernels.h"
+#include "rank.cuh"
 
 namespace srs {
 
@@ -120,21 +121,8 @@ __global__ void cosine_kernel(const float* __restrict__ q, const float* __restri
   const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const int lane = threadIdx.x & 31;
   if (warp >= n) return;
-  const float* v = c + (size_t)warp * dim;
-  double dot = 0.0, n1 = 0.0, n2 = 0.0;
-  for (int k = lane; k < dim; k += 32) {
-    const float a = __ldg(q + k), bb = __ldg(v + k);
-    dot += (double)__fmul_rn(a, bb);
-    n1 += (double)__fmul_rn(a, a);
-    n2 += (double)__fmul_rn(bb, bb);
-  }
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) {
-    dot += __shfl_xor_sync(0xffffffffu, dot, o);
-    n1 += __shfl_xor_sync(0xffffffffu, n1, o);
-    n2 += __shfl_xor_sync(0xffffffffu, n2, o);
-  }
-  if (lane == 0) out[warp] = (float)(dot / (sqrt(n1) * sqrt(n2)));
+  const float r = cosine_warp(q, c + (size_t)warp * dim, dim, lane);
+  if (lane == 0) out[warp] = r;
 }
 
 cudaError_t launch_cosine(const float* q, const float* c, int n, int dim, float* out,
