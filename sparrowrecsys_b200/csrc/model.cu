@@ -7,6 +7,7 @@
 #include <cstdlib>
 #include <cstring>
 #include <atomic>
+#include <initializer_list>
 #include <map>
 #include <mutex>
 #include <string>
@@ -121,6 +122,10 @@ struct Slot {
   int32_t* h_req = nullptr;         // pinned copy of it
 };
 
+// The forward kernel a model runs, chosen when it is created.  din_rt, din_rtp and din_rt64 all read
+// srs_model::din_rt.
+enum class Kernel { ncf, embmlp, embmlp_tc, deepfm, deepfm_tc, deepfm2, din, din_tc, din_rt, din_rtp, din_rt64, dien };
+
 }  // namespace
 
 struct srs_model {
@@ -128,6 +133,7 @@ struct srs_model {
   int device = 0;
   int EP = 0;
   int hist_cols = 0;                // history columns the model reads (T for DIN, 1 for W&D)
+  bool dense_feats = false;         // reads movie_genre / user_genre / numerics (all but NeuralCF and two towers)
   std::vector<void*> owned;
   int* err_flag = nullptr;          // kErrWords device words: [0] srs_predict_device, [1 + i] host slot i.  One word
                                     // per slot: a flag shared by every slot could be copied by slot A, set by
@@ -139,16 +145,10 @@ struct srs_model {
   DinParams din{};
   DienParams dien{};
   DinTcParams din_tc{};
-  bool use_din_tc = false;
   DinRtParams din_rt{};
-  bool use_din_rt = false;
-  bool use_din_rt64 = false;         // din_rt holds the parameters of din_rt64_kernel
-  bool use_din_rtp = false;          // din_rt holds the parameters; the pipelined row-tile kernel runs them
   EmbMlpTcParams emb_tc{};
-  bool use_emb_tc = false;
   DeepFmTcParams fm_tc{};
-  bool use_fm_tc = false;
-  const char* kernel_name = "";
+  Kernel kernel = Kernel::ncf;
   bool no_zero_copy = false;         // SRS_ZERO_COPY_SCORES=0 switches the latency path of srs_predict_host off
   bool zero_copy_scores = false;     // SRS_ZERO_COPY_SCORES=1 (experimental): kernels write the scores
                                      // of a host batch straight into the caller's pinned buffer
@@ -162,6 +162,48 @@ struct srs_model {
 
 namespace {
 inline int* slot_err(srs_model* m, const Slot& s) { return m->err_flag + 1 + (&s - m->slots); }
+
+const char* kernel_name(const srs_model* m) {
+  const bool wide = m->spec.kind == SRS_WIDENDEEP;
+  switch (m->kernel) {
+    case Kernel::ncf: return m->spec.kind == SRS_TWOTOWERS ? "ncf_kernel<two_towers>" : "ncf_kernel<neural_cf_model_1>";
+    case Kernel::embmlp: return wide ? "embmlp_kernel<wide&deep>" : "embmlp_kernel";
+    case Kernel::embmlp_tc: return wide ? "embmlp_tc_kernel<wide&deep>" : "embmlp_tc_kernel";
+    case Kernel::deepfm: return "deepfm_kernel";
+    case Kernel::deepfm_tc: return "deepfm_tc_kernel";
+    case Kernel::deepfm2: return "deepfm2_kernel";
+    case Kernel::din: return "din_kernel";
+    case Kernel::din_tc: return "din_tc_kernel";
+    case Kernel::din_rt: return "din_rt_kernel";
+    case Kernel::din_rtp: return "din_rtp_kernel";
+    case Kernel::din_rt64: return "din_rt64_kernel";
+    case Kernel::dien: return "dien_kernel";
+  }
+  return "";
+}
+
+// A kernel the `*_impl` option can force: the option value, whether the model's shape fits the kernel, and
+// the error when it is forced onto a shape that does not.
+struct Forced {
+  const char* value;
+  Kernel kernel;
+  bool fits;
+  const char* needs;
+};
+
+// m->kernel = `def`, unless the create option `key` (else the environment variable `env`) names one of
+// `forced`; a value that names none of them leaves the default.
+int select_kernel(srs_model* m, const char* key, const char* env, Kernel def, std::initializer_list<Forced> forced) {
+  m->kernel = def;
+  const char* impl = opt(key, env);
+  if (!impl) return SRS_OK;
+  for (const Forced& f : forced)
+    if (!strcmp(impl, f.value)) {
+      if (!f.fits) return fail(SRS_ERR_INVALID, "%s", f.needs);
+      m->kernel = f.kernel;
+    }
+  return SRS_OK;
+}
 }  // namespace
 
 
@@ -210,18 +252,24 @@ struct Builder {
     return t->data;
   }
 
-  float* upload(const std::vector<float>& v) {
+  // device allocation owned by the model
+  void* alloc(size_t bytes) {
     if (status != SRS_OK) return nullptr;
-    float* d = nullptr;
-    size_t bytes = (v.size() ? v.size() : 1) * sizeof(float);
+    void* d = nullptr;
     cudaError_t e = cudaMalloc(&d, bytes);
     if (e != cudaSuccess) {
       status = fail(SRS_ERR_NOMEM, "cudaMalloc(%zu) failed: %s", bytes, cudaGetErrorString(e));
       return nullptr;
     }
     m->owned.push_back(d);
-    if (!v.empty()) {
-      e = cudaMemcpy(d, v.data(), v.size() * sizeof(float), cudaMemcpyHostToDevice);
+    return d;
+  }
+
+  template <class T>
+  T* upload(const std::vector<T>& v) {
+    T* d = static_cast<T*>(alloc((v.size() ? v.size() : 1) * sizeof(T)));
+    if (d && !v.empty()) {
+      cudaError_t e = cudaMemcpy(d, v.data(), v.size() * sizeof(T), cudaMemcpyHostToDevice);
       if (e != cudaSuccess) {
         status = fail(SRS_ERR_CUDA, "cudaMemcpy H2D failed: %s", cudaGetErrorString(e));
         return nullptr;
@@ -301,6 +349,47 @@ std::vector<int> iota_map(int start, int n, int padded) {
 
 void append(std::vector<int>& a, const std::vector<int>& b) { a.insert(a.end(), b.begin(), b.end()); }
 
+// Rows of a reference layer-1 dense/kernel: the first row of each embedding block, in the order the
+// kernels gather the blocks, and the seven numeric rows in NUMERIC_KEYS order.
+struct DenseRows {
+  std::vector<int> emb;
+  int num[7];
+};
+
+// DenseFeatures sorted concat (SURVEY.md 8a row a2): movieGenre1..3, movieId, userGenre1..5, userId
+DenseRows embmlp_rows(int E) {
+  return {{1, 1 + E, 1 + 2 * E, 1 + 3 * E, 5 + 4 * E, 5 + 5 * E, 5 + 6 * E, 5 + 7 * E, 5 + 8 * E, 5 + 9 * E},
+          {0, 1 + 4 * E, 2 + 4 * E, 3 + 4 * E, 4 + 4 * E, 5 + 10 * E, 6 + 10 * E}};
+}
+
+// deep movieId, deep userId
+DenseRows deepfm_rows(int E) { return {{1, 5 + E}, {0, 1 + E, 2 + E, 3 + E, 4 + E, 5 + 2 * E, 6 + 2 * E}}; }
+
+// [user_profile | pooled | candidate | context] (DIN.py:161-162): userGenre1, userId, pooled behaviours,
+// candidate, movieGenre1
+DenseRows din_rows(int E) {
+  const int base = 3 + 4 * E;
+  return {{1, 1 + E, 3 + 2 * E, 3 + 3 * E, base + 1},
+          {base, base + 1 + E, base + 2 + E, base + 3 + E, 0, 1 + 2 * E, 2 + 2 * E}};
+}
+
+// CUDA-core layer-1 row map: every embedding block padded to EP, then the numerics and one zero row
+std::vector<int> layer1_map(const DenseRows& r, int E, int EP) {
+  std::vector<int> map;
+  for (int start : r.emb) append(map, iota_map(start, E, EP));
+  map.insert(map.end(), r.num, r.num + 7);
+  map.push_back(-1);
+  return map;
+}
+
+// [8][pitch] numeric rows of layer 1 (row 7 zero), the fp32 term of the tensor-core kernels
+std::vector<float> pack_w1num(const float* k1, int h0, const DenseRows& r, int pitch) {
+  std::vector<float> w((size_t)8 * pitch, 0.f);
+  for (int n = 0; n < 7; ++n)
+    for (int j = 0; j < h0; ++j) w[(size_t)n * pitch + j] = k1[(size_t)r.num[n] * h0 + j];
+  return w;
+}
+
 // ------------------------------------------------------------------------------------
 int build_ncf(Builder& B) {
   srs_model* m = B.m;
@@ -375,7 +464,6 @@ int build_ncf(Builder& B) {
   if (B.status != SRS_OK) return B.status;
   p.blob = B.upload(blob);
   p.blob_floats = (int)blob.size();
-  m->kernel_name = two ? "ncf_kernel<two_towers>" : "ncf_kernel<neural_cf_model_1>";
   return B.status;
 }
 
@@ -399,14 +487,6 @@ int build_embmlp(Builder& B) {
   }
   p.movie = B.table("movieId_embedding", s.n_movies, E);
   p.user = B.table("userId_embedding", s.n_users, E);
-  // reference row order of dense/kernel: DenseFeatures sorted concat (SURVEY.md 8a row a2)
-  std::vector<int> map;
-  for (int k = 0; k < 3; ++k) append(map, iota_map(1 + k * E, E, EP));         // movieGenre1..3
-  append(map, iota_map(1 + 3 * E, E, EP));                                        // movieId
-  for (int k = 0; k < 5; ++k) append(map, iota_map(5 + 4 * E + k * E, E, EP));   // userGenre1..5
-  append(map, iota_map(5 + 9 * E, E, EP));                                        // userId
-  const int nums[8] = {0, 1 + 4 * E, 2 + 4 * E, 3 + 4 * E, 4 + 4 * E, 5 + 10 * E, 6 + 10 * E, -1};
-  for (int j = 0; j < 8; ++j) map.push_back(nums[j]);
   const float* k1 = B.host("dense/kernel", 7 + 10 * E, h0);
   const float* b1 = B.host("dense/bias", h0, 1);
   const float* k2 = B.host("dense_1/kernel", h0, h1);
@@ -415,7 +495,7 @@ int build_embmlp(Builder& B) {
   const float* k3 = B.host("dense_2/kernel", last_in, 1);
   const float* b3 = B.host("dense_2/bias", 1, 1);
   if (B.status != SRS_OK) return B.status;
-  p.W1 = B.upload(B.permute(k1, h0, map, 128));
+  p.W1 = B.upload(B.permute(k1, h0, layer1_map(embmlp_rows(E), E, EP), 128));
   p.b1 = B.upload(B.padvec(b1, h0, 128));
   p.W2 = B.upload(B.permute(k2, h1, iota_map(0, h0, 128), 128));
   p.b2 = B.upload(B.padvec(b2, h1, 128));
@@ -425,7 +505,6 @@ int build_embmlp(Builder& B) {
   p.b3 = b3[0];
   p.n_movies = s.n_movies; p.n_users = s.n_users; p.n_genres = s.n_genres;
   p.cross_buckets = s.cross_buckets; p.EP = EP;
-  m->kernel_name = wide ? "embmlp_kernel<wide&deep>" : "embmlp_kernel";
   return B.status;
 }
 
@@ -444,11 +523,6 @@ int build_deepfm(Builder& B) {
   p.fm_ugenre = B.table("fm_userGenre1_embedding", s.n_genres, E);
   p.deep_movie = B.table("deep_movieId_embedding", s.n_movies, E);
   p.deep_user = B.table("deep_userId_embedding", s.n_users, E);
-  std::vector<int> map;
-  append(map, iota_map(1, E, EP));            // deep movieId emb
-  append(map, iota_map(5 + E, E, EP));        // deep userId emb
-  const int nums[8] = {0, 1 + E, 2 + E, 3 + E, 4 + E, 5 + 2 * E, 6 + 2 * E, -1};
-  for (int j = 0; j < 8; ++j) map.push_back(nums[j]);
   const float* k1 = B.host("dense/kernel", 7 + 2 * E, h0);
   const float* b1 = B.host("dense/bias", h0, 1);
   const float* k2 = B.host("dense_1/kernel", h0, h1);
@@ -456,7 +530,7 @@ int build_deepfm(Builder& B) {
   const float* k3 = B.host("dense_2/kernel", fm1 + 4 + h1, 1);
   const float* b3 = B.host("dense_2/bias", 1, 1);
   if (B.status != SRS_OK) return B.status;
-  p.W1 = B.upload(B.permute(k1, h0, map, 64));
+  p.W1 = B.upload(B.permute(k1, h0, layer1_map(deepfm_rows(E), E, EP), 64));
   p.b1 = B.upload(B.padvec(b1, h0, 64));
   p.W2 = B.upload(B.permute(k2, h1, iota_map(0, h0, 64), 64));
   p.b2 = B.upload(B.padvec(b2, h1, 64));
@@ -465,7 +539,6 @@ int build_deepfm(Builder& B) {
   p.wdeep = B.upload(B.padvec(k3 + fm1 + 4, h1, 64));
   p.bout = b3[0];
   p.n_movies = s.n_movies; p.n_users = s.n_users; p.n_genres = s.n_genres; p.EP = EP;
-  m->kernel_name = "deepfm_kernel";
   return B.status;
 }
 
@@ -521,7 +594,6 @@ int build_deepfm2(Builder& B) {
   p.wout = B.upload(B.padvec(ok, 1 + P + h1, 1 + P + 16));
   p.bout = ob[0];
   p.n_movies = s.n_movies; p.n_users = s.n_users; p.n_genres = s.n_genres; p.EP = EP;
-  m->kernel_name = "deepfm2_kernel";
   return B.status;
 }
 
@@ -568,17 +640,7 @@ int build_din(Builder& B) {
   p.au_alpha = B.upload(std::vector<float>(alpha, alpha + (size_t)T * A));
   p.au_wout = B.upload(std::vector<float>(auo, auo + A));
   p.au_bout = auob[0];
-  // top kernel rows: [user_profile | pooled | candidate | context] (DIN.py:161-162)
-  const int base = 3 + 4 * E;
-  std::vector<int> map;
-  append(map, iota_map(1, E, EP));               // userGenre1 emb
-  append(map, iota_map(1 + E, E, EP));           // userId emb
-  append(map, iota_map(3 + 2 * E, E, EP));       // pooled behaviours
-  append(map, iota_map(3 + 3 * E, E, EP));       // candidate emb
-  append(map, iota_map(base + 1, E, EP));        // movieGenre1 emb
-  const int nums[8] = {base, base + 1 + E, base + 2 + E, base + 3 + E, 0, 1 + 2 * E, 2 + 2 * E, -1};
-  for (int j = 0; j < 8; ++j) map.push_back(nums[j]);
-  p.W1 = B.upload(B.permute(k1, h0, map, 128));
+  p.W1 = B.upload(B.permute(k1, h0, layer1_map(din_rows(E), E, EP), 128));
   p.b1 = B.upload(B.padvec(b1, h0, 128));
   p.a1 = B.upload(B.padvec(a1, h0, 128));
   p.W2 = B.upload(B.permute(k2, h1, iota_map(0, h0, 128), 64));
@@ -588,7 +650,6 @@ int build_din(Builder& B) {
   p.b3 = b3[0];
   p.n_movies = s.n_movies; p.n_users = s.n_users; p.n_genres = s.n_genres;
   p.T = T; p.EP = EP;
-  m->kernel_name = "din_kernel";
   return B.status;
 }
 
@@ -670,16 +731,11 @@ int build_dien(Builder& B) {
   p.seq = B.upload(q);
   // top kernel rows: [augru | candidate | user_profile | context] (DIEN.py:250); the blocks
   // are DenseFeatures layers, sorted by column name inside (as in DIN)
+  // embedding blocks in DIN's gather order: userGenre1, userId, AUGRU final state, candidate, movieGenre1
   const int up = 2 * E, ctx = 4 * E + 3;
-  std::vector<int> map;
-  append(map, iota_map(up + 1, E, EP));          // userGenre1 emb
-  append(map, iota_map(up + 1 + E, E, EP));      // userId emb
-  append(map, iota_map(0, E, EP));               // AUGRU final state
-  append(map, iota_map(E, E, EP));               // candidate emb
-  append(map, iota_map(ctx + 1, E, EP));         // movieGenre1 emb
-  const int nums[8] = {ctx, ctx + 1 + E, ctx + 2 + E, ctx + 3 + E, up, up + 1 + 2 * E, up + 2 + 2 * E, -1};
-  for (int j = 0; j < 8; ++j) map.push_back(nums[j]);
-  p.W1 = B.upload(B.permute(k1, h0, map, 128));
+  const DenseRows rows = {{up + 1, up + 1 + E, 0, E, ctx + 1},
+                          {ctx, ctx + 1 + E, ctx + 2 + E, ctx + 3 + E, up, up + 1 + 2 * E, up + 2 + 2 * E}};
+  p.W1 = B.upload(B.permute(k1, h0, layer1_map(rows, E, EP), 128));
   p.b1 = B.upload(B.padvec(b1, h0, 128));
   p.a1 = B.upload(B.padvec(a1, h0, 128));
   p.W2 = B.upload(B.permute(k2, h1, iota_map(0, h0, 128), 64));
@@ -689,7 +745,6 @@ int build_dien(Builder& B) {
   p.b3 = b3[0];
   p.n_movies = s.n_movies; p.n_users = s.n_users; p.n_genres = s.n_genres;
   p.T = T; p.EP = EP;
-  m->kernel_name = "dien_kernel";
   return B.status;
 }
 
@@ -717,6 +772,78 @@ void write_sw128(uint8_t* dst, int rows, int kblocks, bool lo_part, F get) {
         }
 }
 
+// Layer-1 embedding weights as hi and lo MMA operands: row = unit j, K = block * width + e, the blocks of
+// `r.emb` in order (zero for j >= h0, e >= E and past the last block).
+void write_w1_image(uint8_t* hi, uint8_t* lo, int kblocks, const float* k1, int h0, const DenseRows& r, int E,
+                    int width) {
+  const int nb = (int)r.emb.size();
+  auto get = [&](int j, int k) -> float {
+    const int b = k / width, e = k - b * width;
+    if (j >= h0 || b >= nb || e >= E) return 0.f;
+    return k1[(size_t)(r.emb[b] + e) * h0 + j];
+  };
+  write_sw128(hi, 128, kblocks, false, get);
+  write_sw128(lo, 128, kblocks, true, get);
+}
+
+// Layer-2 weights W2^T [unit i][k], zero for i >= h1 or k >= h0
+float w2t(const float* k2, int h0, int h1, int i, int k) { return (i < h1 && k < h0) ? k2[(size_t)k * h1 + i] : 0.f; }
+
+void write_w2_image(uint8_t* hi, uint8_t* lo, int kblocks, const float* k2, int h0, int h1) {
+  auto get = [&](int i, int k) { return w2t(k2, h0, h1, i, k); };
+  write_sw128(hi, 128, kblocks, false, get);
+  write_sw128(lo, 128, kblocks, true, get);
+}
+
+// DIN's layer-2 A operand, one 128-row tile per K block: rows 0..63 = hi halves of W2^T, rows 64..127 = lo halves
+void write_w2_stacked(uint8_t* dst, const float* k2, int h0, int h1) {
+  for (int kb = 0; kb < 2; ++kb)
+    for (int r = 0; r < 128; ++r)
+      for (int c = 0; c < 8; ++c)
+        for (int i = 0; i < 8; ++i) {
+          const float x = w2t(k2, h0, h1, r & 63, kb * 64 + c * 8 + i);
+          const uint16_t hb = bf16_rn_bits(x);
+          const uint16_t v = (r < 64) ? hb : bf16_rn_bits(x - u2f((uint32_t)hb << 16));
+          memcpy(dst + (size_t)kb * 16384 + sw128_off(r, c) + i * 2, &v, 2);
+        }
+}
+
+// Activation unit, history side: (Wsub + Wh)^T and Wp^T as [unit j][e] with row pitch `pitch`, zero beyond E
+// (rows of au_dense/kernel are [h-c | h | c | h*c] blocks of E)
+void au_transposed(const float* au, int E, int pitch, std::vector<float>& waT, std::vector<float>& wpT) {
+  const int A = 32;
+  waT.assign((size_t)A * pitch, 0.f);
+  wpT.assign((size_t)A * pitch, 0.f);
+  for (int j = 0; j < A; ++j)
+    for (int e = 0; e < E; ++e) {
+      waT[(size_t)j * pitch + e] = au[(size_t)e * A + j] + au[(size_t)(E + e) * A + j];
+      wpT[(size_t)j * pitch + e] = au[(size_t)(3 * E + e) * A + j];
+    }
+}
+
+// PReLU + Dense(1) of the activation unit folded into two tables per position t < T:
+//   wout_j max(v,0) + alpha_tj wout_j min(v,0) = v P_tj + |v| Q_tj;  put(t, j, P_tj, Q_tj)
+template <class F>
+void fold_pq(const float* alpha, const float* auo, int T, F put) {
+  for (int t = 0; t < T; ++t)
+    for (int j = 0; j < 32; ++j) {
+      const float wo = auo[j], aw = alpha[(size_t)t * 32 + j] * auo[j];
+      put(t, j, 0.5f * (wo + aw), 0.5f * (wo - aw));
+    }
+}
+
+// Tables and vectors build_din uploaded (or borrowed) that the tensor-core DIN kernels read unchanged
+template <class P>
+void copy_din_common(P& p, const DinParams& v1) {
+  p.movie = v1.movie; p.user = v1.user; p.ugenre = v1.ugenre; p.mgenre = v1.mgenre;
+  p.au_wc = v1.au_wc; p.au_b = v1.au_b;
+  p.b1 = v1.b1; p.a1 = v1.a1;
+  p.b2 = v1.b2; p.a2 = v1.a2; p.w3 = v1.w3;
+  p.au_bout = v1.au_bout; p.b3 = v1.b3;
+  p.n_movies = v1.n_movies; p.n_users = v1.n_users; p.n_genres = v1.n_genres;
+  p.T = v1.T;
+}
+
 // Fills m->din_tc from the same reference tensors build_din validated.
 int build_din_tc(Builder& B) {
   srs_model* m = B.m;
@@ -730,91 +857,46 @@ int build_din_tc(Builder& B) {
   const float* k1 = B.host("dense/kernel", 5 * E + 7, h0);
   const float* k2 = B.host("dense_1/kernel", h0, h1);
   if (B.status != SRS_OK) return B.status;
+  const DenseRows rows = din_rows(E);
   // image offsets mirror the constants in din_tc.cu
   const uint32_t IMG_AUB_HI = 0, IMG_AUB_LO = 4096, IMG_W1_HI = 8192, IMG_W1_LO = IMG_W1_HI + 3 * 16384,
                  IMG_W2 = IMG_W1_LO + 3 * 16384, IMG_PQ = IMG_W2 + 2 * 16384;
   const uint32_t kPqStride = 68;
-  const uint32_t bytes = IMG_PQ + (uint32_t)TP * kPqStride * 4u;
-  std::vector<uint8_t> img(bytes, 0);
+  std::vector<uint8_t> img(IMG_PQ + (uint32_t)TP * kPqStride * 4u, 0);
   // activation unit B operand: row j = [ (Wsub+Wh)[e][j], e<32 | Wp[e][j], e<32 ]
-  auto au_get = [&](int j, int k) -> float {
-    const int e = k & 31;
-    if (e >= E) return 0.f;
-    if (k < 32) return au[(size_t)e * A + j] + au[(size_t)(E + e) * A + j];
-    return au[(size_t)(3 * E + e) * A + j];
-  };
+  std::vector<float> waT, wpT;
+  au_transposed(au, E, 32, waT, wpT);
+  auto au_get = [&](int j, int k) -> float { return (k < 32 ? waT : wpT)[(size_t)j * 32 + (k & 31)]; };
   write_sw128(img.data() + IMG_AUB_HI, 32, 1, false, au_get);
   write_sw128(img.data() + IMG_AUB_LO, 32, 1, true, au_get);
   // layer 1 A operand: row = unit j, K = [userGenre1 | userId | pooled | candidate | movieGenre1 | 0] x 32
-  const int base = 3 + 4 * E;
-  const int slot_start[6] = {1, 1 + E, 3 + 2 * E, 3 + 3 * E, base + 1, -1};
-  auto w1_get = [&](int j, int k) -> float {
-    const int slot = k >> 5, e = k & 31;
-    if (j >= h0 || slot >= 5 || e >= E) return 0.f;
-    return k1[(size_t)(slot_start[slot] + e) * h0 + j];
-  };
-  write_sw128(img.data() + IMG_W1_HI, 128, 3, false, w1_get);
-  write_sw128(img.data() + IMG_W1_LO, 128, 3, true, w1_get);
-  // layer 2 A operand: rows 0..63 = hi halves of W2^T, rows 64..127 = lo halves
-  auto w2_raw = [&](int i, int k) -> float { return (i < h1 && k < h0) ? k2[(size_t)k * h1 + i] : 0.f; };
-  {
-    std::vector<uint8_t> hi(2 * 64 * 128), lo(2 * 64 * 128);
-    // build as two 64-row matrices, then interleave into 128-row tiles
-    for (int kb = 0; kb < 2; ++kb)
-      for (int r = 0; r < 128; ++r)
-        for (int c = 0; c < 8; ++c)
-          for (int i = 0; i < 8; ++i) {
-            const float x = w2_raw(r & 63, kb * 64 + c * 8 + i);
-            const uint16_t hb = bf16_rn_bits(x);
-            const uint16_t v = (r < 64) ? hb : bf16_rn_bits(x - u2f((uint32_t)hb << 16));
-            memcpy(img.data() + IMG_W2 + (size_t)kb * 16384 + sw128_off(r, c) + i * 2, &v, 2);
-          }
-  }
-  // PReLU + Dense(1) folded into two tables, one 68-float row per position t (zero beyond T):
-  //   wout_j max(v,0) + alpha_tj wout_j min(v,0) = v P_tj + |v| Q_tj
-  // stored as 16 x (P_2m, P_2m+1, Q_2m, Q_2m+1) so one 128-bit load feeds two packed FMAs
+  write_w1_image(img.data() + IMG_W1_HI, img.data() + IMG_W1_LO, 3, k1, h0, rows, E, 32);
+  write_w2_stacked(img.data() + IMG_W2, k2, h0, h1);
+  // P/Q: one 68-float row per position t (zero beyond T), stored as 16 x (P_2m, P_2m+1, Q_2m, Q_2m+1) so
+  // one 128-bit load feeds two packed FMAs
   float* PQ = reinterpret_cast<float*>(img.data() + IMG_PQ);
-  for (int t = 0; t < T; ++t)
-    for (int j = 0; j < A; ++j) {
-      const float wo = auo[j], aw = alpha[(size_t)t * A + j] * auo[j];
-      float* cell = PQ + (size_t)t * kPqStride + (j >> 1) * 4 + (j & 1);
-      cell[0] = 0.5f * (wo + aw);
-      cell[2] = 0.5f * (wo - aw);
-    }
-  uint8_t* d_img = nullptr;
-  cudaError_t e = cudaMalloc(&d_img, bytes);
-  if (e != cudaSuccess) return fail(SRS_ERR_NOMEM, "cudaMalloc(%u) failed: %s", bytes, cudaGetErrorString(e));
-  m->owned.push_back(d_img);
-  e = cudaMemcpy(d_img, img.data(), bytes, cudaMemcpyHostToDevice);
-  if (e != cudaSuccess) return fail(SRS_ERR_CUDA, "image upload failed: %s", cudaGetErrorString(e));
-  // numerics rows of dense/kernel in NUMERIC_KEYS order
-  const int nrows[7] = {base, base + 1 + E, base + 2 + E, base + 3 + E, 0, 1 + 2 * E, 2 + 2 * E};
-  std::vector<float> w1num(8 * 128, 0.f);
-  for (int n = 0; n < 7; ++n)
-    for (int j = 0; j < h0; ++j) w1num[(size_t)n * 128 + j] = k1[(size_t)nrows[n] * h0 + j];
+  fold_pq(alpha, auo, T, [&](int t, int j, float P, float Q) {
+    float* cell = PQ + (size_t)t * kPqStride + (j >> 1) * 4 + (j & 1);
+    cell[0] = P;
+    cell[2] = Q;
+  });
   DinTcParams& p = m->din_tc;
-  const DinParams& v1 = m->din;                 // reuse tables / vectors uploaded by build_din
-  p.movie = v1.movie; p.user = v1.user; p.ugenre = v1.ugenre; p.mgenre = v1.mgenre;
-  p.image = d_img;
-  p.au_wc = v1.au_wc; p.au_b = v1.au_b;
-  p.b1 = v1.b1; p.a1 = v1.a1; p.w1num = B.upload(w1num);
-  p.b2 = v1.b2; p.a2 = v1.a2; p.w3 = v1.w3;
+  copy_din_common(p, m->din);
+  p.image = B.upload(img);
+  p.w1num = B.upload(pack_w1num(k1, h0, rows, 128));
   for (int j = 0; j < A; ++j) p.au_wout[j] = auo[j];
-  p.au_bout = v1.au_bout; p.b3 = v1.b3;
-  p.n_movies = s.n_movies; p.n_users = s.n_users; p.n_genres = s.n_genres;
-  p.T = T; p.CPR = CPR;
-  int sms = 0;
-  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, m->device);
-  p.num_sms = sms > 0 ? sms : 148;
+  p.CPR = CPR;
+  p.num_sms = m->device_sms;
   return B.status;
 }
 
-// Row-tile DIN kernel (din_rt.cu): pre-split movie table, transposed activation-unit weights,
-// P/Q gate tables and the top-MLP operand images, from the tensors build_din validated.
+// Row-tile DIN kernels, E padded to 32 (din_rt.cu; din_rtp.cu runs the same parameters) or to 64
+// (din_rt64.cu): pre-split movie table, transposed activation-unit weights, P/Q gate tables and the
+// top-MLP operand images, from the tensors build_din validated.
 int build_din_rt(Builder& B) {
   srs_model* m = B.m;
   const srs_spec& s = m->spec;
-  const int E = s.emb_dim, T = s.hist_len, A = 32;
+  const int E = s.emb_dim, EP = m->EP, T = s.hist_len, A = 32;
   const int h0 = s.hidden[0], h1 = s.hidden[1];
   const float* au = B.host("au_dense/kernel", 4 * E, A);
   const float* alpha = B.host("au_prelu/alpha", T, A);
@@ -822,202 +904,78 @@ int build_din_rt(Builder& B) {
   const float* k1 = B.host("dense/kernel", 5 * E + 7, h0);
   const float* k2 = B.host("dense_1/kernel", h0, h1);
   if (B.status != SRS_OK) return B.status;
-  const uint32_t RI_W2 = 0, RI_W1_HI = 32768, RI_W1_LO = RI_W1_HI + 49152, RI_BYTES = RI_W1_LO + 49152;
-  std::vector<uint8_t> img(RI_BYTES, 0);
-  const int base = 3 + 4 * E;
-  const int slot_start[6] = {1, 1 + E, 3 + 2 * E, 3 + 3 * E, base + 1, -1};
-  auto w1_get = [&](int j, int k) -> float {
-    const int slot = k >> 5, e = k & 31;
-    if (j >= h0 || slot >= 5 || e >= E) return 0.f;
-    return k1[(size_t)(slot_start[slot] + e) * h0 + j];
-  };
-  write_sw128(img.data() + RI_W1_HI, 128, 3, false, w1_get);
-  write_sw128(img.data() + RI_W1_LO, 128, 3, true, w1_get);
-  auto w2_raw = [&](int i, int k) -> float { return (i < h1 && k < h0) ? k2[(size_t)k * h1 + i] : 0.f; };
-  for (int kb = 0; kb < 2; ++kb)
-    for (int r = 0; r < 128; ++r)
-      for (int c = 0; c < 8; ++c)
-        for (int i = 0; i < 8; ++i) {
-          const float x = w2_raw(r & 63, kb * 64 + c * 8 + i);
-          const uint16_t hb = bf16_rn_bits(x);
-          const uint16_t v = (r < 64) ? hb : bf16_rn_bits(x - u2f((uint32_t)hb << 16));
-          memcpy(img.data() + RI_W2 + (size_t)kb * 16384 + sw128_off(r, c) + i * 2, &v, 2);
-        }
-  uint8_t* d_img = nullptr;
-  cudaError_t e = cudaMalloc(&d_img, RI_BYTES);
-  if (e != cudaSuccess) return fail(SRS_ERR_NOMEM, "cudaMalloc(%u) failed: %s", RI_BYTES, cudaGetErrorString(e));
-  m->owned.push_back(d_img);
-  e = cudaMemcpy(d_img, img.data(), RI_BYTES, cudaMemcpyHostToDevice);
-  if (e != cudaSuccess) return fail(SRS_ERR_CUDA, "image upload failed: %s", cudaGetErrorString(e));
-  // activation unit: (Wsub + Wh)^T and Wp^T, [unit j][e], zero beyond E
-  std::vector<float> waT(32 * 32, 0.f), wpT(32 * 32, 0.f);
-  for (int j = 0; j < A; ++j)
-    for (int ee = 0; ee < E; ++ee) {
-      waT[(size_t)j * 32 + ee] = au[(size_t)ee * A + j] + au[(size_t)(E + ee) * A + j];
-      wpT[(size_t)j * 32 + ee] = au[(size_t)(3 * E + ee) * A + j];
-    }
-  // PReLU + Dense(1) folded: wout_j max(v,0) + alpha_tj wout_j min(v,0) = v P_tj + |v| Q_tj
-  std::vector<float> pq((size_t)T * 64, 0.f);
-  for (int t = 0; t < T; ++t)
-    for (int j = 0; j < A; ++j) {
-      const float wo = auo[j], aw = alpha[(size_t)t * A + j] * auo[j];
-      pq[(size_t)t * 64 + j] = 0.5f * (wo + aw);
-      pq[(size_t)t * 64 + 32 + j] = 0.5f * (wo - aw);
-    }
-  const int nrows[7] = {base, base + 1 + E, base + 2 + E, base + 3 + E, 0, 1 + 2 * E, 2 + 2 * E};
-  std::vector<float> w1num(8 * 128, 0.f);
-  for (int n = 0; n < 7; ++n)
-    for (int j = 0; j < h0; ++j) w1num[(size_t)n * 128 + j] = k1[(size_t)nrows[n] * h0 + j];
-  // din_rtp: W1^T over K = [userId | pooled | candidate] as a tensor-memory A operand (lane = unit,
-  // one 32-bit column per pair of consecutive k: 48 hi words, then 48 lo words), and the two genre
-  // blocks of dense/kernel folded into fp32 tables G[genre][unit] = emb[genre] . rows (exact: 19 values)
-  std::vector<float> w1t_words((size_t)128 * 96, 0.f);
-  {
-    const int kstart[3] = {1 + E, 3 + 2 * E, 3 + 3 * E};
-    auto w1k = [&](int j, int k) -> float {
-      const int f = k >> 5, ee = k & 31;
-      if (j >= h0 || ee >= E) return 0.f;
-      return k1[(size_t)(kstart[f] + ee) * h0 + j];
-    };
-    uint32_t* words = reinterpret_cast<uint32_t*>(w1t_words.data());
-    for (int j = 0; j < 128; ++j)
-      for (int w = 0; w < 48; ++w) {
-        uint32_t hi = 0, lo = 0;
-        for (int half = 0; half < 2; ++half) {
-          const float x = w1k(j, 2 * w + half);
-          const uint16_t hb = bf16_rn_bits(x);
-          const uint16_t lb = bf16_rn_bits(x - u2f((uint32_t)hb << 16));
-          hi |= (uint32_t)hb << (16 * half);
-          lo |= (uint32_t)lb << (16 * half);
-        }
-        words[(size_t)j * 96 + w] = hi;
-        words[(size_t)j * 96 + 48 + w] = lo;
-      }
-  }
-  std::vector<float> gtab_u((size_t)s.n_genres * 128, 0.f), gtab_m((size_t)s.n_genres * 128, 0.f);
-  {
-    const float* ug = B.host("userGenre1_embedding", s.n_genres, E);
-    const float* mg = B.host("movieGenre1_embedding", s.n_genres, E);
-    if (B.status != SRS_OK) return B.status;
-    for (int g = 0; g < s.n_genres; ++g)
-      for (int j = 0; j < h0; ++j) {
-        double su = 0.0, sm = 0.0;
-        for (int ee = 0; ee < E; ++ee) {
-          su += (double)ug[(size_t)g * E + ee] * (double)k1[(size_t)(1 + ee) * h0 + j];
-          sm += (double)mg[(size_t)g * E + ee] * (double)k1[(size_t)(base + 1 + ee) * h0 + j];
-        }
-        gtab_u[(size_t)g * 128 + j] = (float)su;
-        gtab_m[(size_t)g * 128 + j] = (float)sm;
-      }
-  }
+  const DenseRows rows = din_rows(E);
+  // operand images: W1 has one EP-wide K slot per embedding block (3 or 5 K blocks of 16 KB); the order is
+  // W2 | W1 hi | W1 lo in din_rt.cu and W1 hi | W1 lo | W2 in din_rt64.cu
+  const uint32_t w1_blocks = EP == 32 ? 3 : 5, w1_bytes = w1_blocks * 16384, w2_bytes = 2 * 16384;
+  const uint32_t W1_HI = EP == 32 ? w2_bytes : 0, W1_LO = W1_HI + w1_bytes, W2 = EP == 32 ? 0 : 2 * w1_bytes;
+  std::vector<uint8_t> img(2 * w1_bytes + w2_bytes, 0);
+  write_w1_image(img.data() + W1_HI, img.data() + W1_LO, w1_blocks, k1, h0, rows, E, EP);
+  write_w2_stacked(img.data() + W2, k2, h0, h1);
+  std::vector<float> waT, wpT;
+  au_transposed(au, E, EP, waT, wpT);
+  std::vector<float> pq((size_t)T * 64, 0.f);          // [T][P_t 32 | Q_t 32]
+  fold_pq(alpha, auo, T, [&](int t, int j, float P, float Q) {
+    pq[(size_t)t * 64 + j] = P;
+    pq[(size_t)t * 64 + 32 + j] = Q;
+  });
   DinRtParams& p = m->din_rt;
-  const DinParams& v1 = m->din;                 // tables / vectors uploaded by build_din
-  p.w1_tmem = reinterpret_cast<const uint32_t*>(B.upload(w1t_words));
+  copy_din_common(p, m->din);
+  p.image = B.upload(img);
+  // history rows: [n_movies][EP bf16 hi | EP bf16 lo]
+  void* d_split = B.alloc((size_t)s.n_movies * EP * 4);
+  if (B.status != SRS_OK) return B.status;
+  const cudaError_t e = EP == 32 ? launch_split_table(m->din.movie, d_split, s.n_movies, nullptr)
+                                 : launch_split_table64(m->din.movie, d_split, s.n_movies, nullptr);
+  if (e != cudaSuccess) return fail(SRS_ERR_CUDA, "table split failed: %s", cudaGetErrorString(e));
+  p.movie_split = static_cast<const uint8_t*>(d_split);
+  p.waT = B.upload(waT); p.wpT = B.upload(wpT); p.pq = B.upload(pq);
+  p.w1num = B.upload(pack_w1num(k1, h0, rows, 128));
+  p.rows_per_group = 32;
+  if (EP == 64) p.nch = T > 128 ? 2 : 1;
+  p.num_sms = m->device_sms;
+  if (m->kernel != Kernel::din_rtp) return B.status;
+  // din_rtp: W1^T over K = [userId | pooled | candidate] as a tensor-memory A operand (lane = unit, one 32-bit
+  // column per pair of consecutive k: 48 hi words, then 48 lo words), and the two genre blocks of dense/kernel
+  // folded into fp32 tables G[genre][unit] = emb[genre] . rows (exact: 19 values)
+  std::vector<uint32_t> w1t_words((size_t)128 * 96, 0u);
+  auto w1k = [&](int j, int k) -> float {
+    const int f = k >> 5, ee = k & 31;
+    if (j >= h0 || ee >= E) return 0.f;
+    return k1[(size_t)(rows.emb[1 + f] + ee) * h0 + j];
+  };
+  for (int j = 0; j < 128; ++j)
+    for (int w = 0; w < 48; ++w) {
+      uint32_t hi = 0, lo = 0;
+      for (int half = 0; half < 2; ++half) {
+        const float x = w1k(j, 2 * w + half);
+        const uint16_t hb = bf16_rn_bits(x);
+        const uint16_t lb = bf16_rn_bits(x - u2f((uint32_t)hb << 16));
+        hi |= (uint32_t)hb << (16 * half);
+        lo |= (uint32_t)lb << (16 * half);
+      }
+      w1t_words[(size_t)j * 96 + w] = hi;
+      w1t_words[(size_t)j * 96 + 48 + w] = lo;
+    }
+  const float* ug = B.host("userGenre1_embedding", s.n_genres, E);
+  const float* mg = B.host("movieGenre1_embedding", s.n_genres, E);
+  if (B.status != SRS_OK) return B.status;
+  std::vector<float> gtab_u((size_t)s.n_genres * 128, 0.f), gtab_m((size_t)s.n_genres * 128, 0.f);
+  for (int g = 0; g < s.n_genres; ++g)
+    for (int j = 0; j < h0; ++j) {
+      double su = 0.0, sm = 0.0;
+      for (int ee = 0; ee < E; ++ee) {
+        su += (double)ug[(size_t)g * E + ee] * (double)k1[(size_t)(rows.emb[0] + ee) * h0 + j];
+        sm += (double)mg[(size_t)g * E + ee] * (double)k1[(size_t)(rows.emb[4] + ee) * h0 + j];
+      }
+      gtab_u[(size_t)g * 128 + j] = (float)su;
+      gtab_m[(size_t)g * 128 + j] = (float)sm;
+    }
+  p.w1_tmem = B.upload(w1t_words);
   p.gtab_u = B.upload(gtab_u);
   p.gtab_m = B.upload(gtab_m);
-  // history rows: [n_movies][32 bf16 hi | 32 bf16 lo]
-  void* d_split = nullptr;
-  const size_t split_bytes = (size_t)s.n_movies * 128;
-  e = cudaMalloc(&d_split, split_bytes);
-  if (e != cudaSuccess) return fail(SRS_ERR_NOMEM, "cudaMalloc(%zu) failed: %s", split_bytes, cudaGetErrorString(e));
-  m->owned.push_back(d_split);
-  e = launch_split_table(v1.movie, d_split, s.n_movies, nullptr);
-  if (e != cudaSuccess) return fail(SRS_ERR_CUDA, "table split failed: %s", cudaGetErrorString(e));
-  p.movie = v1.movie; p.movie_split = static_cast<const uint8_t*>(d_split);
-  p.user = v1.user; p.ugenre = v1.ugenre; p.mgenre = v1.mgenre;
-  p.image = d_img;
-  p.waT = B.upload(waT); p.wpT = B.upload(wpT); p.pq = B.upload(pq);
-  p.au_wc = v1.au_wc; p.au_b = v1.au_b;
-  p.b1 = v1.b1; p.a1 = v1.a1; p.w1num = B.upload(w1num);
-  p.b2 = v1.b2; p.a2 = v1.a2; p.w3 = v1.w3;
-  p.au_bout = v1.au_bout; p.b3 = v1.b3;
-  p.n_movies = s.n_movies; p.n_users = s.n_users; p.n_genres = s.n_genres;
-  p.T = T; p.rows_per_group = 32;
-  int sms = 0;
-  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, m->device);
-  p.num_sms = sms > 0 ? sms : 148;
-  return B.status;
-}
-
-// Row-tile DIN kernel for E padded to 64 (din_rt64.cu): pre-split movie table (256-byte rows),
-// transposed activation-unit weights, P/Q gate tables, top-MLP images with one K block per feature.
-int build_din_rt64(Builder& B) {
-  srs_model* m = B.m;
-  const srs_spec& s = m->spec;
-  const int E = s.emb_dim, T = s.hist_len, A = 32;
-  const int h0 = s.hidden[0], h1 = s.hidden[1];
-  const float* au = B.host("au_dense/kernel", 4 * E, A);
-  const float* alpha = B.host("au_prelu/alpha", T, A);
-  const float* auo = B.host("au_out/kernel", A, 1);
-  const float* k1 = B.host("dense/kernel", 5 * E + 7, h0);
-  const float* k2 = B.host("dense_1/kernel", h0, h1);
-  if (B.status != SRS_OK) return B.status;
-  const uint32_t W1HI = 0, W1LO = 81920, W2OFF = 163840, BYTES = 196608;
-  std::vector<uint8_t> img(BYTES, 0);
-  const int base = 3 + 4 * E;
-  const int slot_start[5] = {1, 1 + E, 3 + 2 * E, 3 + 3 * E, base + 1};   // userGenre1, userId, pooled, candidate, movieGenre1
-  auto w1_get = [&](int j, int k) -> float {
-    const int slot = k >> 6, e = k & 63;
-    if (j >= h0 || slot >= 5 || e >= E) return 0.f;
-    return k1[(size_t)(slot_start[slot] + e) * h0 + j];
-  };
-  write_sw128(img.data() + W1HI, 128, 5, false, w1_get);
-  write_sw128(img.data() + W1LO, 128, 5, true, w1_get);
-  auto w2_raw = [&](int i, int k) -> float { return (i < h1 && k < h0) ? k2[(size_t)k * h1 + i] : 0.f; };
-  for (int kb = 0; kb < 2; ++kb)
-    for (int r = 0; r < 128; ++r)
-      for (int c = 0; c < 8; ++c)
-        for (int i = 0; i < 8; ++i) {
-          const float x = w2_raw(r & 63, kb * 64 + c * 8 + i);
-          const uint16_t hb = bf16_rn_bits(x);
-          const uint16_t v = (r < 64) ? hb : bf16_rn_bits(x - u2f((uint32_t)hb << 16));
-          memcpy(img.data() + W2OFF + (size_t)kb * 16384 + sw128_off(r, c) + i * 2, &v, 2);
-        }
-  uint8_t* d_img = nullptr;
-  cudaError_t e = cudaMalloc(&d_img, BYTES);
-  if (e != cudaSuccess) return fail(SRS_ERR_NOMEM, "cudaMalloc(%u) failed: %s", BYTES, cudaGetErrorString(e));
-  m->owned.push_back(d_img);
-  e = cudaMemcpy(d_img, img.data(), BYTES, cudaMemcpyHostToDevice);
-  if (e != cudaSuccess) return fail(SRS_ERR_CUDA, "image upload failed: %s", cudaGetErrorString(e));
-  std::vector<float> waT(32 * 64, 0.f), wpT(32 * 64, 0.f);
-  for (int j = 0; j < A; ++j)
-    for (int ee = 0; ee < E; ++ee) {
-      waT[(size_t)j * 64 + ee] = au[(size_t)ee * A + j] + au[(size_t)(E + ee) * A + j];
-      wpT[(size_t)j * 64 + ee] = au[(size_t)(3 * E + ee) * A + j];
-    }
-  std::vector<float> pq((size_t)T * 64, 0.f);
-  for (int t = 0; t < T; ++t)
-    for (int j = 0; j < A; ++j) {
-      const float wo = auo[j], aw = alpha[(size_t)t * A + j] * auo[j];
-      pq[(size_t)t * 64 + j] = 0.5f * (wo + aw);
-      pq[(size_t)t * 64 + 32 + j] = 0.5f * (wo - aw);
-    }
-  const int nrows[7] = {base, base + 1 + E, base + 2 + E, base + 3 + E, 0, 1 + 2 * E, 2 + 2 * E};
-  std::vector<float> w1num(8 * 128, 0.f);
-  for (int n = 0; n < 7; ++n)
-    for (int j = 0; j < h0; ++j) w1num[(size_t)n * 128 + j] = k1[(size_t)nrows[n] * h0 + j];
-  DinRtParams& p = m->din_rt;
-  const DinParams& v1 = m->din;                 // tables / vectors uploaded (or borrowed) by build_din, pitch 64
-  void* d_split = nullptr;
-  const size_t split_bytes = (size_t)s.n_movies * 256;
-  e = cudaMalloc(&d_split, split_bytes);
-  if (e != cudaSuccess) return fail(SRS_ERR_NOMEM, "cudaMalloc(%zu) failed: %s", split_bytes, cudaGetErrorString(e));
-  m->owned.push_back(d_split);
-  e = launch_split_table64(v1.movie, d_split, s.n_movies, nullptr);
-  if (e != cudaSuccess) return fail(SRS_ERR_CUDA, "table split failed: %s", cudaGetErrorString(e));
-  p.movie = v1.movie; p.movie_split = static_cast<const uint8_t*>(d_split);
-  p.user = v1.user; p.ugenre = v1.ugenre; p.mgenre = v1.mgenre;
-  p.image = d_img;
-  p.waT = B.upload(waT); p.wpT = B.upload(wpT); p.pq = B.upload(pq);
-  p.au_wc = v1.au_wc; p.au_b = v1.au_b;
-  p.b1 = v1.b1; p.a1 = v1.a1; p.w1num = B.upload(w1num);
-  p.b2 = v1.b2; p.a2 = v1.a2; p.w3 = v1.w3;
-  p.au_bout = v1.au_bout; p.b3 = v1.b3;
-  p.n_movies = s.n_movies; p.n_users = s.n_users; p.n_genres = s.n_genres;
-  p.T = T; p.rows_per_group = 32; p.nch = T > 128 ? 2 : 1;
-  int sms = 0;
-  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, m->device);
-  p.num_sms = sms > 0 ? sms : 148;
+  const cudaError_t ea = setup_din_rtp_attributes();
+  if (ea != cudaSuccess) return fail(SRS_ERR_CUDA, "din_rtp attribute setup failed: %s", cudaGetErrorString(ea));
   return B.status;
 }
 
@@ -1029,44 +987,19 @@ int build_embmlp_tc(Builder& B) {
   const float* k1 = B.host("dense/kernel", 7 + 10 * E, h0);
   const float* k2 = B.host("dense_1/kernel", h0, h1);
   if (B.status != SRS_OK) return B.status;
-  // K = slot * 12 + e; slot order of the kernel's gather: movieGenre1..3, movieId, userGenre1..5, userId
-  int slot_start[10];
-  for (int k = 0; k < 3; ++k) slot_start[k] = 1 + k * E;
-  slot_start[3] = 1 + 3 * E;
-  for (int k = 0; k < 5; ++k) slot_start[4 + k] = 5 + 4 * E + k * E;
-  slot_start[9] = 5 + 9 * E;
-  auto w1_get = [&](int j, int k) -> float {
-    const int slot = k / 12, e = k - slot * 12;
-    if (j >= h0 || slot >= 10 || e >= E) return 0.f;
-    return k1[(size_t)(slot_start[slot] + e) * h0 + j];
-  };
-  auto w2_get = [&](int j, int k) -> float { return (j < h1 && k < h0) ? k2[(size_t)k * h1 + j] : 0.f; };
+  const DenseRows rows = embmlp_rows(E);
   std::vector<uint8_t> img(131072, 0);
-  write_sw128(img.data() + 0, 128, 2, false, w1_get);
-  write_sw128(img.data() + 32768, 128, 2, true, w1_get);
-  write_sw128(img.data() + 65536, 128, 2, false, w2_get);
-  write_sw128(img.data() + 98304, 128, 2, true, w2_get);
-  uint8_t* d_img = nullptr;
-  cudaError_t e = cudaMalloc(&d_img, img.size());
-  if (e != cudaSuccess) return fail(SRS_ERR_NOMEM, "cudaMalloc failed: %s", cudaGetErrorString(e));
-  m->owned.push_back(d_img);
-  e = cudaMemcpy(d_img, img.data(), img.size(), cudaMemcpyHostToDevice);
-  if (e != cudaSuccess) return fail(SRS_ERR_CUDA, "image upload failed: %s", cudaGetErrorString(e));
-  const int nrows[7] = {0, 1 + 4 * E, 2 + 4 * E, 3 + 4 * E, 4 + 4 * E, 5 + 10 * E, 6 + 10 * E};
-  std::vector<float> w1num(8 * 128, 0.f);
-  for (int n = 0; n < 7; ++n)
-    for (int j = 0; j < h0; ++j) w1num[(size_t)n * 128 + j] = k1[(size_t)nrows[n] * h0 + j];
+  write_w1_image(img.data() + 0, img.data() + 32768, 2, k1, h0, rows, E, 12);     // K = block * 12 + e
+  write_w2_image(img.data() + 65536, img.data() + 98304, 2, k2, h0, h1);
   EmbMlpTcParams& p = m->emb_tc;
   const EmbMlpParams& v1 = m->emb;
   for (int k = 0; k < 8; ++k) p.genre[k] = v1.genre[k];
   p.movie = v1.movie; p.user = v1.user;
-  p.image = d_img;
+  p.image = B.upload(img);
   p.b1 = v1.b1; p.b2 = v1.b2; p.w3 = v1.w3; p.wide = v1.wide; p.b3 = v1.b3;
-  p.w1num = B.upload(w1num);
+  p.w1num = B.upload(pack_w1num(k1, h0, rows, 128));
   p.n_movies = s.n_movies; p.n_users = s.n_users; p.n_genres = s.n_genres; p.cross_buckets = s.cross_buckets;
-  int sms = 0;
-  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, m->device);
-  p.num_sms = sms > 0 ? sms : 148;
+  p.num_sms = m->device_sms;
   return B.status;
 }
 
@@ -1078,41 +1011,21 @@ int build_deepfm_tc(Builder& B) {
   const float* k1 = B.host("dense/kernel", 7 + 2 * E, h0);
   const float* k2 = B.host("dense_1/kernel", h0, h1);
   if (B.status != SRS_OK) return B.status;
-  auto w1_get = [&](int j, int k) -> float {        // K = [deep movieId emb (16) | deep userId emb (16) | 0]
-    if (j >= h0 || k >= 32) return 0.f;
-    const int e = k & 15;
-    if (e >= E) return 0.f;
-    return k1[(size_t)((k < 16 ? 1 : 5 + E) + e) * h0 + j];
-  };
-  auto w2_get = [&](int j, int k) -> float { return (j < h1 && k < h0) ? k2[(size_t)k * h1 + j] : 0.f; };
+  const DenseRows rows = deepfm_rows(E);
   std::vector<uint8_t> img(65536, 0);
-  write_sw128(img.data() + 0, 128, 1, false, w1_get);
-  write_sw128(img.data() + 16384, 128, 1, true, w1_get);
-  write_sw128(img.data() + 32768, 128, 1, false, w2_get);
-  write_sw128(img.data() + 49152, 128, 1, true, w2_get);
-  uint8_t* d_img = nullptr;
-  cudaError_t e = cudaMalloc(&d_img, img.size());
-  if (e != cudaSuccess) return fail(SRS_ERR_NOMEM, "cudaMalloc failed: %s", cudaGetErrorString(e));
-  m->owned.push_back(d_img);
-  e = cudaMemcpy(d_img, img.data(), img.size(), cudaMemcpyHostToDevice);
-  if (e != cudaSuccess) return fail(SRS_ERR_CUDA, "image upload failed: %s", cudaGetErrorString(e));
-  const int nrows[7] = {0, 1 + E, 2 + E, 3 + E, 4 + E, 5 + 2 * E, 6 + 2 * E};
-  std::vector<float> w1num(8 * 64, 0.f);
-  for (int n = 0; n < 7; ++n)
-    for (int j = 0; j < h0; ++j) w1num[(size_t)n * 64 + j] = k1[(size_t)nrows[n] * h0 + j];
+  write_w1_image(img.data() + 0, img.data() + 16384, 1, k1, h0, rows, E, 16);     // K = [movieId 16 | userId 16 | 0]
+  write_w2_image(img.data() + 32768, img.data() + 49152, 1, k2, h0, h1);
   DeepFmTcParams& p = m->fm_tc;
   const DeepFmParams& v1 = m->fm;
   p.fm_movie = v1.fm_movie; p.fm_user = v1.fm_user; p.fm_mgenre = v1.fm_mgenre; p.fm_ugenre = v1.fm_ugenre;
   p.deep_movie = v1.deep_movie; p.deep_user = v1.deep_user;
-  p.image = d_img;
+  p.image = B.upload(img);
   p.b1 = v1.b1; p.b2 = v1.b2; p.first = v1.first; p.wdeep = v1.wdeep;
-  p.w1num = B.upload(w1num);
+  p.w1num = B.upload(pack_w1num(k1, h0, rows, 64));
   for (int d = 0; d < 4; ++d) p.wdot[d] = v1.wdot[d];
   p.bout = v1.bout;
   p.n_movies = s.n_movies; p.n_users = s.n_users; p.n_genres = s.n_genres;
-  int sms = 0;
-  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, m->device);
-  p.num_sms = sms > 0 ? sms : 148;
+  p.num_sms = m->device_sms;
   return B.status;
 }
 
@@ -1136,9 +1049,7 @@ int check_batch(const srs_model* m, const srs_batch* b) {
   if (b->B < 0) return fail(SRS_ERR_INVALID, "negative batch size");
   if (b->B == 0) return SRS_OK;
   if (!b->movie_id || !b->user_id) return fail(SRS_ERR_INVALID, "movie_id / user_id are required");
-  const int k = m->spec.kind;
-  const bool dense_feats = !(k == SRS_NEURALCF || k == SRS_TWOTOWERS);
-  if (dense_feats && (!b->movie_genre || !b->user_genre || !b->numerics))
+  if (m->dense_feats && (!b->movie_genre || !b->user_genre || !b->numerics))
     return fail(SRS_ERR_INVALID, "movie_genre / user_genre / numerics are required for this model");
   if (m->hist_cols > 0) {
     if (!b->hist && !b->hist16) return fail(SRS_ERR_INVALID, "hist is required for this model");
@@ -1152,26 +1063,19 @@ int check_batch(const srs_model* m, const srs_batch* b) {
 
 int launch(srs_model* m, const BatchView& v, cudaStream_t stream) {
   cudaError_t e = cudaSuccess;
-  switch (m->spec.kind) {
-    case SRS_NEURALCF:
-    case SRS_TWOTOWERS: e = launch_ncf(m->ncf, v, stream); break;
-    case SRS_EMBEDDINGMLP:
-    case SRS_WIDENDEEP:
-      e = m->use_emb_tc ? launch_embmlp_tc(m->emb_tc, v, stream) : launch_embmlp(m->emb, v, stream);
-      break;
-    case SRS_DEEPFM:
-      e = m->use_fm_tc ? launch_deepfm_tc(m->fm_tc, v, stream) : launch_deepfm(m->fm, v, stream);
-      break;
-    case SRS_DEEPFM_V2: e = launch_deepfm2(m->fm2, v, stream); break;
-    case SRS_DIN:
-      e = m->use_din_rt64 ? launch_din_rt64(m->din_rt, v, stream)
-          : m->use_din_rtp ? launch_din_rtp(m->din_rt, v, stream)
-          : m->use_din_rt ? launch_din_rt(m->din_rt, v, stream)
-          : m->use_din_tc ? launch_din_tc(m->din_tc, v, stream)
-                          : launch_din(m->din, v, stream);
-      break;
-    case SRS_DIEN: e = launch_dien(m->dien, v, stream); break;
-    default: return fail(SRS_ERR_INVALID, "unknown model kind");
+  switch (m->kernel) {
+    case Kernel::ncf: e = launch_ncf(m->ncf, v, stream); break;
+    case Kernel::embmlp: e = launch_embmlp(m->emb, v, stream); break;
+    case Kernel::embmlp_tc: e = launch_embmlp_tc(m->emb_tc, v, stream); break;
+    case Kernel::deepfm: e = launch_deepfm(m->fm, v, stream); break;
+    case Kernel::deepfm_tc: e = launch_deepfm_tc(m->fm_tc, v, stream); break;
+    case Kernel::deepfm2: e = launch_deepfm2(m->fm2, v, stream); break;
+    case Kernel::din: e = launch_din(m->din, v, stream); break;
+    case Kernel::din_tc: e = launch_din_tc(m->din_tc, v, stream); break;
+    case Kernel::din_rt: e = launch_din_rt(m->din_rt, v, stream); break;
+    case Kernel::din_rtp: e = launch_din_rtp(m->din_rt, v, stream); break;
+    case Kernel::din_rt64: e = launch_din_rt64(m->din_rt, v, stream); break;
+    case Kernel::dien: e = launch_dien(m->dien, v, stream); break;
   }
   if (e != cudaSuccess) return fail(SRS_ERR_CUDA, "kernel launch failed: %s", cudaGetErrorString(e));
   return SRS_OK;
@@ -1184,8 +1088,7 @@ struct PackedLayout {
   size_t movie, user, hist, mg, ug, num, total;
 };
 PackedLayout packed_layout(const srs_model* m, size_t B, bool narrow_hist = false) {
-  const int k = m->spec.kind;
-  const bool dense_feats = !(k == SRS_NEURALCF || k == SRS_TWOTOWERS);
+  const bool dense_feats = m->dense_feats;
   PackedLayout L{};
   size_t off = 0;
   L.movie = off; off += B * 4;
@@ -1197,6 +1100,33 @@ PackedLayout packed_layout(const srs_model* m, size_t B, bool narrow_hist = fals
   L.num = off; off += dense_feats ? B * 7 * 4 : 0;
   L.total = off;
   return L;
+}
+
+// Kernel view of a batch staged at `d` in the packed order; the caller sets the outputs and the error word.
+BatchView packed_view(const srs_model* m, const uint8_t* d, const PackedLayout& L, int B) {
+  BatchView v{};
+  v.B = B; v.hist_stride = m->hist_cols;
+  v.movie_id = reinterpret_cast<const int32_t*>(d + L.movie);
+  v.user_id = reinterpret_cast<const int32_t*>(d + L.user);
+  v.hist = reinterpret_cast<const int32_t*>(d + L.hist);
+  v.movie_genre = reinterpret_cast<const int32_t*>(d + L.mg);
+  v.user_genre = reinterpret_cast<const int32_t*>(d + L.ug);
+  v.numerics = reinterpret_cast<const float*>(d + L.num);
+  return v;
+}
+
+// Kernel view of a batch whose arrays are on the device already (after check_batch); the caller sets the
+// outputs.
+int device_view(srs_model* m, const srs_batch* b, BatchView& v) {
+  if (m->hist_cols > 0 && !b->hist)
+    return fail(SRS_ERR_INVALID, "device batches carry int32 history ids (hist16 is for host batches)");
+  CUDA_TRY(cudaSetDevice(m->device));
+  v = BatchView{};
+  v.B = b->B; v.hist_stride = b->hist_stride;
+  v.movie_id = b->movie_id; v.user_id = b->user_id; v.hist = b->hist;
+  v.movie_genre = b->movie_genre; v.user_genre = b->user_genre; v.numerics = b->numerics;
+  v.err_flag = m->err_flag;
+  return SRS_OK;
 }
 
 int ensure_slot(srs_model* m, Slot& s, int B) {
@@ -1231,8 +1161,6 @@ int stage_and_launch(srs_model* m, Slot& s, const srs_batch* b, bool want_logits
   if (rc != SRS_OK) return rc;
   if (b->B == 0) return SRS_OK;
   const size_t B = (size_t)b->B;
-  const int k = m->spec.kind;
-  const bool dense_feats = !(k == SRS_NEURALCF || k == SRS_TWOTOWERS);
   const bool narrow = m->hist_cols > 0 && b->hist16 != nullptr;
   const PackedLayout L = packed_layout(m, B, narrow);
   uint8_t* d = s.d_block;
@@ -1242,7 +1170,7 @@ int stage_and_launch(srs_model* m, Slot& s, const srs_batch* b, bool want_logits
     packed = packed && b->hist_stride == m->hist_cols &&
              (narrow ? reinterpret_cast<const uint8_t*>(b->hist16)
                      : reinterpret_cast<const uint8_t*>(b->hist)) == h0 + L.hist;
-  if (dense_feats)
+  if (m->dense_feats)
     packed = packed && reinterpret_cast<const uint8_t*>(b->movie_genre) == h0 + L.mg &&
              reinterpret_cast<const uint8_t*>(b->user_genre) == h0 + L.ug &&
              reinterpret_cast<const uint8_t*>(b->numerics) == h0 + L.num;
@@ -1261,28 +1189,31 @@ int stage_and_launch(srs_model* m, Slot& s, const srs_batch* b, bool want_logits
                                    (size_t)m->hist_cols * es, B, cudaMemcpyHostToDevice, s.stream));
       }
     }
-    if (dense_feats) {
+    if (m->dense_feats) {
       CUDA_TRY(cudaMemcpyAsync(d + L.mg, b->movie_genre, B * 3 * 4, cudaMemcpyHostToDevice, s.stream));
       CUDA_TRY(cudaMemcpyAsync(d + L.ug, b->user_genre, B * 5 * 4, cudaMemcpyHostToDevice, s.stream));
       CUDA_TRY(cudaMemcpyAsync(d + L.num, b->numerics, B * 7 * 4, cudaMemcpyHostToDevice, s.stream));
     }
   }
-  BatchView v{};
-  v.B = b->B; v.hist_stride = m->hist_cols;
-  v.movie_id = reinterpret_cast<const int32_t*>(d + L.movie);
-  v.user_id = reinterpret_cast<const int32_t*>(d + L.user);
-  v.hist = reinterpret_cast<const int32_t*>(d + L.hist);
+  BatchView v = packed_view(m, d, L, b->B);
   if (narrow) {
     CUDA_TRY(launch_widen_u16(reinterpret_cast<const uint16_t*>(d + L.hist), s.d_hist32,
                               (int64_t)B * m->hist_cols, s.stream));
     v.hist = s.d_hist32;
   }
-  v.movie_genre = reinterpret_cast<const int32_t*>(d + L.mg);
-  v.user_genre = reinterpret_cast<const int32_t*>(d + L.ug);
-  v.numerics = reinterpret_cast<const float*>(d + L.num);
   v.probs = probs_out ? probs_out : s.d_probs;
   v.logits = want_logits ? (logits_out ? logits_out : s.d_logits) : nullptr; v.err_flag = slot_err(m, s);
   return launch(m, v, s.stream);
+}
+
+// device-visible alias of a host pointer if it is pinned (page-locked) memory, else nullptr
+float* pinned_alias(float* p) {
+  if (!p) return nullptr;
+  cudaPointerAttributes at{};
+  if (cudaPointerGetAttributes(&at, p) == cudaSuccess && at.type == cudaMemoryTypeHost && at.devicePointer)
+    return static_cast<float*>(at.devicePointer);
+  cudaGetLastError();                                   // pageable memory: not an error
+  return nullptr;
 }
 
 int enqueue_host(srs_model* m, Slot& s, const srs_batch* b, float* probs, float* logits,
@@ -1291,14 +1222,7 @@ int enqueue_host(srs_model* m, Slot& s, const srs_batch* b, float* probs, float*
   // Experimental (SRS_ZERO_COPY_SCORES=1): a pinned output buffer is device-addressable under
   // unified addressing, so the kernel can write the 4 B per row over PCIe itself and the
   // device-to-host copy - one driver call and one copy-engine operation per batch - goes away.
-  float* direct = nullptr;
-  if (m->zero_copy_scores && b && b->B > 0) {
-    cudaPointerAttributes at{};
-    if (cudaPointerGetAttributes(&at, probs) == cudaSuccess && at.type == cudaMemoryTypeHost && at.devicePointer)
-      direct = static_cast<float*>(at.devicePointer);
-    else
-      cudaGetLastError();                                 // pageable memory: not an error, use the copy
-  }
+  float* direct = m->zero_copy_scores && b && b->B > 0 ? pinned_alias(probs) : nullptr;   // pageable: the copy
   int rc = stage_and_launch(m, s, b, logits != nullptr, direct);
   if (rc != SRS_OK) return rc;
   if (b->B == 0) return SRS_OK;
@@ -1362,6 +1286,33 @@ int wait_done(srs_model* m, Slot& s) {
   return SRS_OK;
 }
 
+// Top k of the n scores in s.d_probs into top_idx / top_scores.  The ranking kernel writes the k positions
+// and scores into pinned host memory and then the completion record the caller spins on: no device-to-host
+// copy, no stream synchronise.
+int rank_scores(srs_model* m, Slot& s, int n, int k, int32_t* top_idx, float* top_scores) {
+  int rc = ensure_done(s, k);
+  if (rc != SRS_OK) return rc;
+  if (k > 0 && n > s.rank_capacity) {
+    cudaFree(s.d_rank);
+    s.d_rank = nullptr;
+    s.rank_capacity = 0;
+    const int cap = s.capacity;     // >= n: the scores are in this slot's staging
+    CUDA_TRY(cudaMalloc(&s.d_rank, (size_t)cap * 8 + topk_scratch_bytes(cap) + 256));
+    s.rank_capacity = cap;
+  }
+  int32_t* r_idx = s.h_res;
+  float* r_top = reinterpret_cast<float*>(s.h_res + s.res_capacity);
+  void* scratch = s.d_rank ? s.d_rank + (size_t)s.rank_capacity * 8 : nullptr;
+  s.seq += 1;
+  CUDA_TRY(launch_topk_done(s.d_probs, n, k, r_idx, r_top, scratch, slot_err(m, s), s.h_done, s.seq, s.stream));
+  rc = wait_done(m, s);
+  if (k > 0) {
+    memcpy(top_idx, r_idx, (size_t)k * 4);
+    if (top_scores) memcpy(top_scores, r_top, (size_t)k * 4);
+  }
+  return rc;
+}
+
 }  // namespace
 
 // ======================================================================================
@@ -1413,6 +1364,7 @@ int srs_model_create(const srs_spec* spec, const srs_tensor* tensors, int32_t n_
   m->EP = round_ep(spec->emb_dim);
   m->hist_cols = (spec->kind == SRS_DIN || spec->kind == SRS_DIEN) ? spec->hist_len
                  : spec->kind == SRS_WIDENDEEP ? 1 : 0;
+  m->dense_feats = !(spec->kind == SRS_NEURALCF || spec->kind == SRS_TWOTOWERS);
   m->bytes_per_inf = bytes_per_inference(*spec);
   Builder B{m};
   for (int i = 0; i < n_tensors; ++i)
@@ -1420,99 +1372,60 @@ int srs_model_create(const srs_spec* spec, const srs_tensor* tensors, int32_t n_
   int rc;
   switch (spec->kind) {
     case SRS_NEURALCF:
-    case SRS_TWOTOWERS: rc = build_ncf(B); break;
+    case SRS_TWOTOWERS: m->kernel = Kernel::ncf; rc = build_ncf(B); break;
     case SRS_EMBEDDINGMLP:
     case SRS_WIDENDEEP: {
       rc = build_embmlp(B);
-      // tensor-core path for the reference shape (E <= 12); SRS_EMBMLP_IMPL=cudacore|tc overrides
-      const char* impl_c = opt("embmlp_impl", "SRS_EMBMLP_IMPL");
-      const std::string impl_s = impl_c ? impl_c : "";
-      const char* impl = impl_c ? impl_s.c_str() : nullptr;
-      const bool fits = m->EP == 12;
-      bool want = fits;
-      if (impl && !strcmp(impl, "cudacore")) want = false;
-      if (impl && !strcmp(impl, "tc")) {
-        if (!fits && rc == SRS_OK) rc = fail(SRS_ERR_INVALID, "SRS_EMBMLP_IMPL=tc needs emb_dim <= 12");
-        want = true;
-      }
-      if (rc == SRS_OK && want) {
-        rc = build_embmlp_tc(B);
-        if (rc == SRS_OK) {
-          m->use_emb_tc = true;
-          m->kernel_name = spec->kind == SRS_WIDENDEEP ? "embmlp_tc_kernel<wide&deep>" : "embmlp_tc_kernel";
-        }
-      }
+      // tensor cores for the reference shape (E <= 12)
+      const bool tc = m->EP == 12;
+      if (rc == SRS_OK)
+        rc = select_kernel(m, "embmlp_impl", "SRS_EMBMLP_IMPL", tc ? Kernel::embmlp_tc : Kernel::embmlp,
+                           {{"cudacore", Kernel::embmlp, true, nullptr},
+                            {"tc", Kernel::embmlp_tc, tc, "SRS_EMBMLP_IMPL=tc needs emb_dim <= 12"}});
       break;
     }
     case SRS_DEEPFM: {
       rc = build_deepfm(B);
-      // tensor-core deep MLP when emb_dim pads to 16; SRS_DEEPFM_IMPL=cudacore|tc overrides
-      const char* impl_c = opt("deepfm_impl", "SRS_DEEPFM_IMPL");
-      const std::string impl_s = impl_c ? impl_c : "";
-      const char* impl = impl_c ? impl_s.c_str() : nullptr;
-      const bool fits = m->EP == 16;
-      bool want = fits;
-      if (impl && !strcmp(impl, "cudacore")) want = false;
-      if (impl && !strcmp(impl, "tc")) {
-        if (!fits && rc == SRS_OK) rc = fail(SRS_ERR_INVALID, "SRS_DEEPFM_IMPL=tc needs 12 < emb_dim <= 16");
-        want = true;
-      }
-      if (rc == SRS_OK && want) {
-        rc = build_deepfm_tc(B);
-        if (rc == SRS_OK) { m->use_fm_tc = true; m->kernel_name = "deepfm_tc_kernel"; }
-      }
+      // tensor-core deep MLP when emb_dim pads to 16
+      const bool tc = m->EP == 16;
+      if (rc == SRS_OK)
+        rc = select_kernel(m, "deepfm_impl", "SRS_DEEPFM_IMPL", tc ? Kernel::deepfm_tc : Kernel::deepfm,
+                           {{"cudacore", Kernel::deepfm, true, nullptr},
+                            {"tc", Kernel::deepfm_tc, tc, "SRS_DEEPFM_IMPL=tc needs 12 < emb_dim <= 16"}});
       break;
     }
-    case SRS_DEEPFM_V2: rc = build_deepfm2(B); break;
-    case SRS_DIEN: rc = build_dien(B); break;
+    case SRS_DEEPFM_V2: m->kernel = Kernel::deepfm2; rc = build_deepfm2(B); break;
+    case SRS_DIEN: m->kernel = Kernel::dien; rc = build_dien(B); break;
     default: {
       rc = build_din(B);
-      // kernel selection (SRS_DIN_IMPL=cudacore|tc|rt overrides; tc / rt fail loudly on an unsupported shape):
-      //   rt  row-tile kernels: E padded to 32 and T in 9..64 (din_rt), E padded to 64 and T in 9..256 (din_rt64)
-      //   tc  per-pair tensor-core kernel, E padded to 32 and T in 9..128
-      const char* impl_c = opt("din_impl", "SRS_DIN_IMPL");
-      const std::string impl_s = impl_c ? impl_c : "";
-      const char* impl = impl_c ? impl_s.c_str() : nullptr;
-      const bool fits_tc = m->EP == 32 && spec->hist_len <= 128;
-      const bool fits_rt32 = m->EP == 32 && spec->hist_len <= 64;
-      const bool fits_rt64 = m->EP == 64 && spec->hist_len <= 256;
-      const bool fits_rt = fits_rt32 || fits_rt64;
-      bool want_rt = fits_rt && spec->hist_len > 8;
-      bool want_tc = !want_rt && fits_tc && spec->hist_len > 8;
-      if (impl && !strcmp(impl, "cudacore")) want_rt = want_tc = false;
-      if (impl && !strcmp(impl, "tc")) {
-        if (!fits_tc && rc == SRS_OK) rc = fail(SRS_ERR_INVALID, "SRS_DIN_IMPL=tc needs 16 < emb_dim <= 32 and hist_len <= 128");
-        want_tc = true; want_rt = false;
-      }
-      const bool want_rtp = impl && !strcmp(impl, "rtp");       // pipelined row-tile kernel (din_rtp.cu)
-      if (want_rtp) {
-        if (!fits_rt32 && rc == SRS_OK)
-          rc = fail(SRS_ERR_INVALID, "SRS_DIN_IMPL=rtp needs 16 < emb_dim <= 32 and hist_len <= 64");
-        want_rt = true; want_tc = false;
-      }
-      if (impl && !strcmp(impl, "rt")) {
-        if (!fits_rt && rc == SRS_OK)
-          rc = fail(SRS_ERR_INVALID, "SRS_DIN_IMPL=rt needs 16 < emb_dim <= 32 and hist_len <= 64, or 32 < emb_dim <= 64 and hist_len <= 256");
-        want_rt = true; want_tc = false;
-      }
-      if (rc == SRS_OK && want_tc) {
-        rc = build_din_tc(B);
-        if (rc == SRS_OK) { m->use_din_tc = true; m->kernel_name = "din_tc_kernel"; }
-      }
-      if (rc == SRS_OK && want_rt && fits_rt32) {
-        rc = build_din_rt(B);
-        if (rc == SRS_OK) { m->use_din_rt = true; m->kernel_name = "din_rt_kernel"; }
-        if (rc == SRS_OK && want_rtp) {
-          cudaError_t ea = setup_din_rtp_attributes();
-          if (ea != cudaSuccess) rc = fail(SRS_ERR_CUDA, "din_rtp attribute setup failed: %s", cudaGetErrorString(ea));
-          m->use_din_rt = false; m->use_din_rtp = true; m->kernel_name = "din_rtp_kernel";
-        }
-      }
-      if (rc == SRS_OK && want_rt && fits_rt64) {
-        rc = build_din_rt64(B);
-        if (rc == SRS_OK) { m->use_din_rt64 = true; m->kernel_name = "din_rt64_kernel"; }
-      }
+      // rt: row-tile kernels, E padded to 32 and T in 9..64 (din_rt), E padded to 64 and T in 9..256 (din_rt64);
+      // tc: per-pair tensor-core kernel, E padded to 32 and T in 9..128.  Forced, tc and rt also take T <= 8;
+      // rtp (the pipelined row-tile kernel, din_rtp.cu) runs only when forced.
+      const int T = spec->hist_len;
+      const bool tc = m->EP == 32 && T <= 128, rt32 = m->EP == 32 && T <= 64, rt64 = m->EP == 64 && T <= 256;
+      const Kernel rt = rt64 ? Kernel::din_rt64 : Kernel::din_rt;
+      const Kernel def = T <= 8 ? Kernel::din : (rt32 || rt64) ? rt : tc ? Kernel::din_tc : Kernel::din;
+      if (rc == SRS_OK)
+        rc = select_kernel(m, "din_impl", "SRS_DIN_IMPL", def,
+                           {{"cudacore", Kernel::din, true, nullptr},
+                            {"tc", Kernel::din_tc, tc, "SRS_DIN_IMPL=tc needs 16 < emb_dim <= 32 and hist_len <= 128"},
+                            {"rtp", Kernel::din_rtp, rt32, "SRS_DIN_IMPL=rtp needs 16 < emb_dim <= 32 and hist_len <= 64"},
+                            {"rt", rt, rt32 || rt64,
+                             "SRS_DIN_IMPL=rt needs 16 < emb_dim <= 32 and hist_len <= 64, "
+                             "or 32 < emb_dim <= 64 and hist_len <= 256"}});
       break;
+    }
+  }
+  // the tensor-core and row-tile kernels read operand images built from the validated reference tensors
+  if (rc == SRS_OK) {
+    switch (m->kernel) {
+      case Kernel::embmlp_tc: rc = build_embmlp_tc(B); break;
+      case Kernel::deepfm_tc: rc = build_deepfm_tc(B); break;
+      case Kernel::din_tc: rc = build_din_tc(B); break;
+      case Kernel::din_rt:
+      case Kernel::din_rtp:
+      case Kernel::din_rt64: rc = build_din_rt(B); break;
+      default: break;
     }
   }
   if (rc == SRS_OK) {
@@ -1566,14 +1479,10 @@ int srs_predict_device(srs_model* m, const srs_batch* b, float* probs, float* lo
   if (rc != SRS_OK) return rc;
   if (!probs) return fail(SRS_ERR_INVALID, "probs is null");
   if (b->B == 0) return SRS_OK;
-  if (m->hist_cols > 0 && !b->hist)
-    return fail(SRS_ERR_INVALID, "device batches carry int32 history ids (hist16 is for host batches)");
-  CUDA_TRY(cudaSetDevice(m->device));
-  BatchView v{};
-  v.B = b->B; v.hist_stride = b->hist_stride;
-  v.movie_id = b->movie_id; v.user_id = b->user_id; v.hist = b->hist;
-  v.movie_genre = b->movie_genre; v.user_genre = b->user_genre; v.numerics = b->numerics;
-  v.probs = probs; v.logits = logits; v.err_flag = m->err_flag;
+  BatchView v;
+  rc = device_view(m, b, v);
+  if (rc != SRS_OK) return rc;
+  v.probs = probs; v.logits = logits;
   return launch(m, v, static_cast<cudaStream_t>(stream));
 }
 
@@ -1610,15 +1519,11 @@ int srs_predict_device_gather(srs_model* m, const srs_batch* b, srs_gather* gg, 
   if (!gather_connected(g)) return fail(SRS_ERR_INVALID, "srs_gather_connect has not been called");
   if (gather_device(g) != m->device) return fail(SRS_ERR_INVALID, "gather object lives on another device");
   if (b->B < 1 || b->B > gather_slice_rows(g)) return fail(SRS_ERR_INVALID, "batch rows must be in 1..slice_rows");
-  if (m->hist_cols > 0 && !b->hist)
-    return fail(SRS_ERR_INVALID, "device batches carry int32 history ids (hist16 is for host batches)");
-  CUDA_TRY(cudaSetDevice(m->device));
-  BatchView v{};
-  v.B = b->B; v.hist_stride = b->hist_stride;
-  v.movie_id = b->movie_id; v.user_id = b->user_id; v.hist = b->hist;
-  v.movie_genre = b->movie_genre; v.user_genre = b->user_genre; v.numerics = b->numerics;
-  v.logits = nullptr; v.err_flag = m->err_flag;
-  const bool in_kernel = m->spec.kind == SRS_DIN && (m->use_din_rtp || m->use_din_rt) ;   // kernels ending in gather_signal_tail()
+  BatchView v;
+  rc = device_view(m, b, v);
+  if (rc != SRS_OK) return rc;
+  // kernels ending in gather_signal_tail()
+  const bool in_kernel = m->kernel == Kernel::din_rt || m->kernel == Kernel::din_rtp;
   gather_begin_step(g, v, in_kernel);
   rc = launch(m, v, static_cast<cudaStream_t>(stream));
   if (rc != SRS_OK) return rc;
@@ -1649,16 +1554,6 @@ int srs_gather_copy_scores(srs_gather* gg, float* dst, int32_t dst_on_host, void
                            dst_on_host ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice,
                            static_cast<cudaStream_t>(stream)));
   return SRS_OK;
-}
-
-// device-visible alias of a host pointer if it is pinned (page-locked) memory, else nullptr
-static float* pinned_alias(float* p) {
-  if (!p) return nullptr;
-  cudaPointerAttributes at{};
-  if (cudaPointerGetAttributes(&at, p) == cudaSuccess && at.type == cudaMemoryTypeHost && at.devicePointer)
-    return static_cast<float*>(at.devicePointer);
-  cudaGetLastError();                                   // pageable memory: not an error
-  return nullptr;
 }
 
 int srs_predict_host(srs_model* m, const srs_batch* b, float* probs, float* logits) {
@@ -1736,7 +1631,7 @@ int srs_model_status(srs_model* m) {
   if (!m) return fail(SRS_ERR_INVALID, "null model");
   CUDA_TRY(cudaSetDevice(m->device));
   CUDA_TRY(cudaDeviceSynchronize());
-  if (m->use_din_rtp) {                              // a protocol error in din_rtp_kernel ends the launch, see rtp_wait
+  if (m->kernel == Kernel::din_rtp) {                // a protocol error in din_rtp_kernel ends the launch, see rtp_wait
     int aborted = 0;
     unsigned long long rec[4] = {0, 0, 0, 0};
     CUDA_TRY(take_din_rtp_abort(&aborted, rec));
@@ -1744,7 +1639,7 @@ int srs_model_status(srs_model* m) {
       return fail(SRS_ERR_CUDA, "din_rtp_kernel: an mbarrier wait timed out (wait code %llu, block %llu, thread %llu, "
                   "parity %llu); the scores of that launch are invalid", rec[0], rec[1], rec[2], rec[3]);
   }
-  if (m->spec.kind == SRS_DIN) {                     // -DRT64_WATCHDOG builds of din_rt64.cu only
+  if (m->kernel == Kernel::din_rt64) {               // -DRT64_WATCHDOG builds of din_rt64.cu only
     int n = 0;
     unsigned long long rec[64];
     CUDA_TRY(take_din_rt64_abort(&n, rec));
@@ -1770,16 +1665,21 @@ int srs_model_status(srs_model* m) {
 
 int64_t srs_model_bytes_per_inference(const srs_model* m) { return m ? m->bytes_per_inf : 0; }
 
-const char* srs_model_kernel_name(const srs_model* m) { return m ? m->kernel_name : ""; }
+const char* srs_model_kernel_name(const srs_model* m) { return m ? kernel_name(m) : ""; }
 
 int srs_model_set_sm_limit(srs_model* m, int32_t n_sms) {
   if (!m) return fail(SRS_ERR_INVALID, "null model");
   const int n = (n_sms <= 0 || n_sms > m->device_sms) ? m->device_sms : n_sms;
   std::lock_guard<std::mutex> lock(m->mu);
-  m->din_rt.num_sms = n;
-  m->din_tc.num_sms = n;
-  m->emb_tc.num_sms = n;
-  m->fm_tc.num_sms = n;
+  switch (m->kernel) {
+    case Kernel::din_rt:
+    case Kernel::din_rtp:
+    case Kernel::din_rt64: m->din_rt.num_sms = n; break;
+    case Kernel::din_tc: m->din_tc.num_sms = n; break;
+    case Kernel::embmlp_tc: m->emb_tc.num_sms = n; break;
+    case Kernel::deepfm_tc: m->fm_tc.num_sms = n; break;
+    default: break;                                  // the CUDA-core kernels take no SM limit
+  }
   return SRS_OK;
 }
 
@@ -1831,29 +1731,7 @@ int srs_rank_host(srs_model* m, const srs_batch* b, int32_t k, int32_t* top_idx,
   if (n == 0) return SRS_OK;
   if (k > n) k = n;
   if (k > 0 && !top_idx) return fail(SRS_ERR_INVALID, "top_idx is null");
-  rc = ensure_done(s, k);
-  if (rc != SRS_OK) return rc;
-  if (k > 0 && n > s.rank_capacity) {
-    cudaFree(s.d_rank);
-    s.d_rank = nullptr;
-    s.rank_capacity = 0;
-    const int cap = s.capacity;     // >= n after stage_and_launch
-    CUDA_TRY(cudaMalloc(&s.d_rank, (size_t)cap * 8 + topk_scratch_bytes(cap) + 256));
-    s.rank_capacity = cap;
-  }
-  // the ranking kernel writes the k positions / scores into pinned host memory and then the completion
-  // record the caller spins on: no device-to-host copy, no stream synchronise
-  int32_t* r_idx = s.h_res;
-  float* r_top = reinterpret_cast<float*>(s.h_res + s.res_capacity);
-  void* scratch = s.d_rank ? s.d_rank + (size_t)s.rank_capacity * 8 : nullptr;
-  s.seq += 1;
-  CUDA_TRY(launch_topk_done(s.d_probs, n, k, r_idx, r_top, scratch, slot_err(m, s), s.h_done, s.seq, s.stream));
-  rc = wait_done(m, s);
-  if (k > 0) {
-    memcpy(top_idx, r_idx, (size_t)k * 4);
-    if (top_scores) memcpy(top_scores, r_top, (size_t)k * 4);
-  }
-  return rc;
+  return rank_scores(m, s, n, k, top_idx, top_scores);
 }
 
 int srs_model_set_movie_features(srs_model* m, int32_t n_movies, const int32_t* genres, const float* numerics) {
@@ -1882,9 +1760,7 @@ int srs_rank_user_host(srs_model* m, const srs_user_row* user, const int32_t* ca
                        int32_t* top_idx, float* top_scores, float* probs) {
   if (!m) return fail(SRS_ERR_INVALID, "null model");
   if (!user || (n > 0 && !cand) || n < 0 || k < 0) return fail(SRS_ERR_INVALID, "bad argument");
-  const int kind = m->spec.kind;
-  const bool dense_feats = !(kind == SRS_NEURALCF || kind == SRS_TWOTOWERS);
-  if (dense_feats && !m->movie_feats)
+  if (m->dense_feats && !m->movie_feats)
     return fail(SRS_ERR_INVALID, "this model reads movie features: call srs_model_set_movie_features first");
   const int hc = m->hist_cols;
   if (user->n_hist < 0 || user->n_hist > hc || (user->n_hist > 0 && !user->hist))
@@ -1900,8 +1776,6 @@ int srs_rank_user_host(srs_model* m, const srs_user_row* user, const int32_t* ca
   if (n > s.req_capacity || !s.d_req) {
     cudaFree(s.d_req);
     if (s.h_req) cudaFreeHost(s.h_req);
-    if (s.h_done) cudaFreeHost(s.h_done);
-    if (s.h_res) cudaFreeHost(s.h_res);
     s.d_req = nullptr; s.h_req = nullptr; s.req_capacity = 0;
     const size_t words = 16 + (size_t)hc + (size_t)s.capacity;
     CUDA_TRY(cudaMalloc(&s.d_req, words * 4));
@@ -1918,20 +1792,11 @@ int srs_rank_user_host(srs_model* m, const srs_user_row* user, const int32_t* ca
   // one small copy: (9 + T + n) words instead of n full feature rows.  (Letting the assemble kernel read the
   // pinned block over PCIe itself was measured slower: every row re-reads the user part from host memory.)
   CUDA_TRY(cudaMemcpyAsync(s.d_req, s.h_req, (9 + (size_t)hc + (size_t)n) * 4, cudaMemcpyHostToDevice, s.stream));
-  rc = ensure_done(s, k);
-  if (rc != SRS_OK) return rc;
   const PackedLayout L = packed_layout(m, (size_t)n);
   uint8_t* d = s.d_block;
-  BatchView v{};
-  v.B = n; v.hist_stride = hc;
-  v.movie_id = reinterpret_cast<const int32_t*>(d + L.movie);
-  v.user_id = reinterpret_cast<const int32_t*>(d + L.user);
-  v.hist = reinterpret_cast<const int32_t*>(d + L.hist);
-  v.movie_genre = reinterpret_cast<const int32_t*>(d + L.mg);
-  v.user_genre = reinterpret_cast<const int32_t*>(d + L.ug);
-  v.numerics = reinterpret_cast<const float*>(d + L.num);
+  BatchView v = packed_view(m, d, L, n);
   v.probs = s.d_probs; v.logits = nullptr; v.err_flag = slot_err(m, s);
-  CUDA_TRY(launch_assemble_request(s.d_req, m->movie_feats, m->movie_feats_rows, n, hc, dense_feats ? 1 : 0,
+  CUDA_TRY(launch_assemble_request(s.d_req, m->movie_feats, m->movie_feats_rows, n, hc, m->dense_feats ? 1 : 0,
                                    reinterpret_cast<int32_t*>(d + L.movie), reinterpret_cast<int32_t*>(d + L.user),
                                    reinterpret_cast<int32_t*>(d + L.hist), reinterpret_cast<int32_t*>(d + L.mg),
                                    reinterpret_cast<int32_t*>(d + L.ug), reinterpret_cast<float*>(d + L.num),
@@ -1939,27 +1804,7 @@ int srs_rank_user_host(srs_model* m, const srs_user_row* user, const int32_t* ca
   rc = launch(m, v, s.stream);
   if (rc != SRS_OK) return rc;
   if (probs) CUDA_TRY(cudaMemcpyAsync(probs, s.d_probs, (size_t)n * 4, cudaMemcpyDeviceToHost, s.stream));
-  if (k > 0 && n > s.rank_capacity) {
-    cudaFree(s.d_rank);
-    s.d_rank = nullptr;
-    s.rank_capacity = 0;
-    const int cap = s.capacity;
-    CUDA_TRY(cudaMalloc(&s.d_rank, (size_t)cap * 8 + topk_scratch_bytes(cap) + 256));
-    s.rank_capacity = cap;
-  }
-  // positions and scores are written into pinned host memory by the ranking kernel itself, followed by the
-  // completion record
-  int32_t* r_idx = s.h_res;
-  float* r_top = reinterpret_cast<float*>(s.h_res + s.res_capacity);
-  void* scratch = s.d_rank ? s.d_rank + (size_t)s.rank_capacity * 8 : nullptr;
-  s.seq += 1;
-  CUDA_TRY(launch_topk_done(s.d_probs, n, k, r_idx, r_top, scratch, slot_err(m, s), s.h_done, s.seq, s.stream));
-  rc = wait_done(m, s);
-  if (k > 0) {
-    memcpy(top_idx, r_idx, (size_t)k * 4);
-    if (top_scores) memcpy(top_scores, r_top, (size_t)k * 4);
-  }
-  return rc;
+  return rank_scores(m, s, n, k, top_idx, top_scores);
 }
 
 int srs_debug_din_trace(srs_model* m, int32_t enable, uint64_t* out40) {
@@ -1969,16 +1814,19 @@ int srs_debug_din_trace(srs_model* m, int32_t enable, uint64_t* out40) {
   m->din_rt.trace = enable;
   if (out40) {
     CUDA_TRY(cudaDeviceSynchronize());
-    if (m->use_din_rtp) CUDA_TRY(read_din_rtp_trace(reinterpret_cast<unsigned long long*>(out40)));
-    else if (m->use_din_rt) CUDA_TRY(read_din_rt_trace(reinterpret_cast<unsigned long long*>(out40)));
-    else CUDA_TRY(read_din_tc_trace(reinterpret_cast<unsigned long long*>(out40)));
+    unsigned long long* out = reinterpret_cast<unsigned long long*>(out40);
+    switch (m->kernel) {
+      case Kernel::din_rtp: CUDA_TRY(read_din_rtp_trace(out)); break;
+      case Kernel::din_rt: CUDA_TRY(read_din_rt_trace(out)); break;
+      default: CUDA_TRY(read_din_tc_trace(out)); break;
+    }
   }
   return SRS_OK;
 }
 
 int srs_debug_din_timeline(srs_model* m, uint64_t* out512) {   /* 12 x 64 values */
   if (!m || !out512) return fail(SRS_ERR_INVALID, "null argument");
-  if (!m->use_din_rtp) return fail(SRS_ERR_INVALID, "the per-tile timeline exists for din_rtp_kernel only");
+  if (m->kernel != Kernel::din_rtp) return fail(SRS_ERR_INVALID, "the per-tile timeline exists for din_rtp_kernel only");
   CUDA_TRY(cudaSetDevice(m->device));
   CUDA_TRY(cudaDeviceSynchronize());
   CUDA_TRY(read_din_rtp_timeline(reinterpret_cast<unsigned long long*>(out512)));
